@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the HybridVAE hot path (BASELINE.json metric: train users/sec & eval top-K users/sec; % of TC/HBM roofline).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c3] [--precision bf16|fp32]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c3] [--precision bf16|fp32] [--dump-outputs DIR]
     python bench.py --impl reference ...      # the reference's CPU path (oracle port) on the host cores
 
 Default workload = BASELINE.json configs[2] (C3): 1M users x 200k items, d = 768, 4,096 users per GPU and step -- the
@@ -39,7 +39,7 @@ DESC = {"c1": "Appliances-shaped synthetic", "c2": "All_Beauty-shaped synthetic"
 def parse_args():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=50)
+    ap.add_argument("--steps", type=int, default=50, help="timed steps (at least 1)")
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--workload", default="c3", choices=["c1", "c2", "c3"])
@@ -51,7 +51,12 @@ def parse_args():
     ap.add_argument("--no-eval", action="store_true")
     ap.add_argument("--no-extras", action="store_true")
     ap.add_argument("--no-graph", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed (losses, updated weights) as DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 def peaks():
@@ -307,8 +312,26 @@ def build_train(name, args, dev, world, rank, batch_override=0):
     return x
 
 
-def measure_train(x, W, K, dev, world, rank, flush_buf, lib):
-    """W warm-up steps, then K timed steps (per-step CUDA events, L2 flushed in between) and K back-to-back steps."""
+def step_outputs(x, w1_sample=1 << 22):
+    """What the most recent training step hands its caller: the three losses and the updated weights under the reference's
+    tensor names.  encoder.0.weight ([h0, N], 480 MB at C3) is reduced to a fixed sample of `w1_sample` flat positions of
+    its [h0, N] shape, drawn from a seeded generator (`encoder.0.weight.sample`); every other tensor is written whole."""
+    out = {"losses": np.asarray(x.trainer.last_losses(), dtype=np.float32)}
+    lay, arena = x.model.layout, x.model.arena.data
+    for k in lay.reference_keys():
+        v = lay.view(arena, k)
+        if k == "encoder.0.weight" and v.numel() > w1_sample:
+            pos = np.sort(np.random.default_rng(0).integers(0, v.numel(), w1_sample))
+            r, c = torch.from_numpy(pos // v.shape[1]).to(v.device), torch.from_numpy(pos % v.shape[1]).to(v.device)
+            out[k + ".sample"] = v[r, c].cpu().numpy()
+        else:
+            out[k] = v.cpu().numpy()
+    return out
+
+
+def measure_train(x, W, K, dev, world, rank, flush_buf, lib, dump_dir=None):
+    """W warm-up steps, then K timed steps (per-step CUDA events, L2 flushed in between) and K back-to-back steps.
+    dump_dir: rank 0 writes step_outputs() of the last timed step there (before the back-to-back steps)."""
     for s in range(W):
         x.step(s)
     barrier(dev, world)
@@ -318,6 +341,15 @@ def measure_train(x, W, K, dev, world, rank, flush_buf, lib):
     barrier(dev, world)
     t1 = time.perf_counter()
     launches = lib.launches - l0
+    if dump_dir is not None:
+        if world > 1:       # per-rank partial sums of the losses -> the global batch's (as train_on_batch returns them)
+            import torch.distributed as dist
+            dist.all_reduce(x.model.engine.loss_out)
+        if rank == 0:
+            Path(dump_dir).mkdir(parents=True, exist_ok=True)
+            for name, a in step_outputs(x).items():
+                np.save(Path(dump_dir) / f"{name}.npy", a)
+        barrier(dev, world)
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for s in range(K):
@@ -742,7 +774,7 @@ def main():
     parity = dp_parity(x, args, dev, world, rank) if world > 1 else None
 
     clocks = ClockSampler(local) if rank == 0 else None
-    r = measure_train(x, W, K, dev, world, rank, flush_buf, lib)
+    r = measure_train(x, W, K, dev, world, rank, flush_buf, lib, args.dump_outputs)
     clk = clocks.stop(*r["wall"]) if clocks else None
     kernels, span_avg, roofline = kernel_spans(x, W, K, flush_buf, pk, world, r["ms_per_step"], args)
     e2e = measure_e2e(x, K, dev, world, rank, flush_buf)

@@ -1,5 +1,7 @@
 import sys
-sys.path[:0]=['/root/repo','/root/repo/recommendation-system_b200']
+from pathlib import Path
+ROOT = Path(__file__).resolve().parents[1]
+sys.path[:0] = [str(ROOT), str(ROOT / "recommendation-system_b200")]
 import torch
 from hvae_b200 import _cabi
 lib=_cabi.lib()
