@@ -177,6 +177,13 @@ size_t hvae_mask_topk_chunks(int n_rows, int N);
 int hvae_mask_topk(float* S, int64_t lds, int n_rows, int N, int item_offset, const int64_t* indptr,
                    const int32_t* indices, const int32_t* rows, int exclude_seen, int K, float* cand_val, int32_t* cand_idx,
                    float* out_val, int32_t* out_idx, void* stream);
+/* The same with per-row item allow-sets: allow is [F, allow_stride_words] bitmaps over global item ids (bit i set = item i may
+ * be returned, allow_stride_words >= ceil((item_offset + N) / 32)), allow_of_row [n_rows] picks a row's bitmap (-1 =
+ * unrestricted).  allow == NULL is hvae_mask_topk.  Slots a row cannot fill hold (-inf, -1). */
+int hvae_mask_topk_filtered(float* S, int64_t lds, int n_rows, int N, int item_offset, const int64_t* indptr,
+                            const int32_t* indices, const int32_t* rows, int exclude_seen, const uint32_t* allow,
+                            int64_t allow_stride_words, const int32_t* allow_of_row, int K, float* cand_val, int32_t* cand_idx,
+                            float* out_val, int32_t* out_idx, void* stream);
 int hvae_topk_merge(const float* cval, const int32_t* cidx, int n_rows, int GK, int K, float* out_val, int32_t* out_idx,
                     void* stream);
 /* The same merge over the blocks of an all-gather, read in place: rank g's K candidates of row r are at
@@ -208,6 +215,12 @@ size_t hvae_tc_topk_splits(int B, int N);
 int hvae_tc_score_topk(const void* U, int ldu, int B, const void* E, int lde, int N, int d, int item_offset,
                        const int64_t* indptr, const int32_t* indices, const int32_t* rows, int K, float* cand_val,
                        int32_t* cand_idx, void* stream);
+/* The same with per-row item allow-sets (bitmaps as in hvae_mask_topk_filtered, over global ids: a shard's item_offset need
+ * not be a multiple of 32).  allow == NULL is hvae_tc_score_topk.  Slots a row cannot fill hold (-inf, -1). */
+int hvae_tc_score_topk_filtered(const void* U, int ldu, int B, const void* E, int lde, int N, int d, int item_offset,
+                                const int64_t* indptr, const int32_t* indices, const int32_t* rows,
+                                const uint32_t* allow, int64_t allow_stride_words, const int32_t* allow_of_row,
+                                int K, float* cand_val, int32_t* cand_idx, void* stream);
 
 /* Backward through the scores: O[b,:] = sum_i softmax(S_b)_i E_i with S recomputed on the tensor cores
  * (autograd of model.py:198,281; E is a frozen buffer, no dE).  lse from hvae_tc_score_lse.

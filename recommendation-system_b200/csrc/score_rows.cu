@@ -362,12 +362,17 @@ constexpr int kTopkSeg = 8;          // 512-byte row segments per trip of the sc
 // segment finds the lanes, four shuffles bring the lane's scores to the whole warp, insertion is warp-uniform.
 // The first trip doubles as a probe: the K-th largest of the 32 per-lane maxima has K scores at or above it, so it is a
 // valid threshold before the first insertion (about rank 40 of the trip's 1024 scores: most of the warm-up is skipped).
+// FILTER: row r may only return items whose bit is set in allow[allow_of_row[r]] (-1: unrestricted).  The allow bits of a
+// trip's scores are fetched with the scores and applied when the trip is consumed (a disallowed score becomes -inf), so the
+// scan keeps its single read of S and its loads in flight; entries left at -inf are written with id -1.
+template <bool FILTER>
 __global__ void __launch_bounds__(kTopkWarps * 32) mask_topk_kernel(float* __restrict__ S, int64_t lds, int n_rows, int N,
                                                                     int item_offset, const int64_t* __restrict__ indptr,
                                                                     const int32_t* __restrict__ indices,
                                                                     const int32_t* __restrict__ rows, int exclude_seen, int K,
                                                                     int n_chunks, int chunk_len, float* __restrict__ out_val,
-                                                                    int32_t* __restrict__ out_idx) {
+                                                                    int32_t* __restrict__ out_idx, const uint32_t* __restrict__ allow,
+                                                                    int64_t allow_stride, const int32_t* __restrict__ allow_of_row) {
     pdl_prologue();
     __shared__ float sv_all[kTopkWarps][kMaxK];
     __shared__ int si_all[kTopkWarps][kMaxK];
@@ -394,14 +399,51 @@ __global__ void __launch_bounds__(kTopkWarps * 32) mask_topk_kernel(float* __res
     const int c1v = cs + ((c1 - cs) / 4) * 4;
     const float4 ninf = make_float4(-INFINITY, -INFINITY, -INFINITY, -INFINITY);
     auto fetch = [&](int base) { const int c = base + lane * 4; return (base < c1v && c < c1v) ? *reinterpret_cast<const float4*>(row + c) : ninf; };
+    const uint32_t* arow = nullptr;
+    if constexpr (FILTER) {
+        const int f = allow_of_row[r];
+        if (f >= 0) arow = allow + (size_t)f * allow_stride;
+    }
+    auto allowed = [&](int c) { const int g = item_offset + c; return !arow || ((__ldg(arow + (g >> 5)) >> (g & 31)) & 1u); };
+    // allow bits of the 4 scores of each segment of a trip, packed 4 per segment (all set when unrestricted)
+    auto fetch_allow = [&](int base) {
+        uint32_t m = 0xFFFFFFFFu;
+        if (arow) {
+            m = 0;
+#pragma unroll
+            for (int q = 0; q < kTopkSeg; ++q) {
+                const int c = base + q * 128 + lane * 4, g = item_offset + c;
+                if (base < c1v && c < c1v) {     // g + 3 < item_offset + N: the second word exists whenever it is needed
+                    const uint32_t lo = __ldg(arow + (g >> 5)), hi = (g & 31) > 28 ? __ldg(arow + (g >> 5) + 1) : 0u;
+                    m |= (__funnelshift_r(lo, hi, g & 31) & 0xFu) << (4 * q);
+                }
+            }
+        }
+        return m;
+    };
     float4 cur[kTopkSeg], nxt[kTopkSeg];
+    uint32_t cur_allow = 0, nxt_allow = 0;
 #pragma unroll
     for (int q = 0; q < kTopkSeg; ++q) cur[q] = fetch(cs + q * 128);
-    top.offer(lane < head ? row[c0 + lane] : -INFINITY, lane < head ? item_offset + c0 + lane : -1);
+    if constexpr (FILTER) cur_allow = fetch_allow(cs);
+    {
+        const bool h = lane < head && (!FILTER || allowed(c0 + lane));
+        top.offer(h ? row[c0 + lane] : -INFINITY, h ? item_offset + c0 + lane : -1);
+    }
     bool probe = K <= 32 && c1v - cs >= kTopkSeg * 128;
     for (int base = cs; base < c1v; base += kTopkSeg * 128) {
 #pragma unroll
         for (int q = 0; q < kTopkSeg; ++q) nxt[q] = fetch(base + kTopkSeg * 128 + q * 128);
+        if constexpr (FILTER) {
+            nxt_allow = fetch_allow(base + kTopkSeg * 128);
+#pragma unroll
+            for (int q = 0; q < kTopkSeg; ++q) {
+                if (!((cur_allow >> (4 * q)) & 1u)) cur[q].x = -INFINITY;
+                if (!((cur_allow >> (4 * q + 1)) & 1u)) cur[q].y = -INFINITY;
+                if (!((cur_allow >> (4 * q + 2)) & 1u)) cur[q].z = -INFINITY;
+                if (!((cur_allow >> (4 * q + 3)) & 1u)) cur[q].w = -INFINITY;
+            }
+        }
         float mq[kTopkSeg];
 #pragma unroll
         for (int q = 0; q < kTopkSeg; ++q) mq[q] = fmaxf(fmaxf(cur[q].x, cur[q].y), fmaxf(cur[q].z, cur[q].w));
@@ -445,9 +487,20 @@ __global__ void __launch_bounds__(kTopkWarps * 32) mask_topk_kernel(float* __res
         }
 #pragma unroll
         for (int q = 0; q < kTopkSeg; ++q) cur[q] = nxt[q];
+        if constexpr (FILTER) cur_allow = nxt_allow;
     }
-    { const int c = c1v + lane; top.offer(c < c1 ? row[c] : -INFINITY, c < c1 ? item_offset + c : -1); }    // <= 3 tail columns
-    top.store(out_val + ((size_t)r * n_chunks + ch) * K, out_idx + ((size_t)r * n_chunks + ch) * K);
+    {   // <= 3 tail columns
+        const int c = c1v + lane;
+        const bool t = c < c1 && (!FILTER || allowed(c));
+        top.offer(t ? row[c] : -INFINITY, t ? item_offset + c : -1);
+    }
+    float* ov = out_val + ((size_t)r * n_chunks + ch) * K;
+    int32_t* oi = out_idx + ((size_t)r * n_chunks + ch) * K;
+    top.store(ov, oi);
+    if constexpr (FILTER) {      // (each lane rereads the slots it wrote)
+        for (int e = lane; e < K; e += 32)
+            if (ov[e] == -INFINITY) oi[e] = -1;
+    }
 }
 
 // Merge G candidate lists per row (item-sharded evaluation, SURVEY.md §8e) -> top K.  Candidate j of row r sits at
@@ -658,10 +711,9 @@ size_t hvae_mask_topk_chunks(int n_rows, int N) {
     return (size_t)nc;
 }
 
-// scratch cand_val / cand_idx: [n_rows, hvae_mask_topk_chunks(n_rows, N) * K] (may be NULL when that is 1)
-int hvae_mask_topk(float* S, int64_t lds, int n_rows, int N, int item_offset, const int64_t* indptr, const int32_t* indices,
-                   const int32_t* rows, int exclude_seen, int K, float* cand_val, int32_t* cand_idx, float* out_val, int32_t* out_idx,
-                   void* stream) {
+static int mask_topk(float* S, int64_t lds, int n_rows, int N, int item_offset, const int64_t* indptr, const int32_t* indices,
+                     const int32_t* rows, int exclude_seen, const uint32_t* allow, int64_t allow_stride, const int32_t* allow_of_row,
+                     int K, float* cand_val, int32_t* cand_idx, float* out_val, int32_t* out_idx, void* stream) {
     HVAE_REQUIRE(K >= 1 && K <= kMaxK, "mask_topk: K=%d outside [1,%d]", K, kMaxK);
     if (n_rows == 0) return 0;
     int nc, len;
@@ -670,15 +722,44 @@ int hvae_mask_topk(float* S, int64_t lds, int n_rows, int N, int item_offset, co
     const int64_t units = (int64_t)n_rows * nc;
     float* cv = nc == 1 ? out_val : cand_val;
     int32_t* ci = nc == 1 ? out_idx : cand_idx;
-    launch_pdl(mask_topk_kernel, (unsigned)((units + kTopkWarps - 1) / kTopkWarps), kTopkWarps * 32, 0, (cudaStream_t)stream, S, lds, n_rows, N,
-               item_offset, indptr, indices, rows, exclude_seen, K, nc, len, cv, ci);
-    HVAE_LAUNCH_CHECK("mask_topk");
+    const unsigned blocks = (unsigned)((units + kTopkWarps - 1) / kTopkWarps);
+    if (allow)
+        launch_pdl(mask_topk_kernel<true>, blocks, kTopkWarps * 32, 0, (cudaStream_t)stream, S, lds, n_rows, N, item_offset, indptr, indices,
+                   rows, exclude_seen, K, nc, len, cv, ci, allow, allow_stride, allow_of_row);
+    else
+        launch_pdl(mask_topk_kernel<false>, blocks, kTopkWarps * 32, 0, (cudaStream_t)stream, S, lds, n_rows, N, item_offset, indptr, indices,
+                   rows, exclude_seen, K, nc, len, cv, ci, (const uint32_t*)nullptr, (int64_t)0, (const int32_t*)nullptr);
+    HVAE_LAUNCH_CHECK(allow ? "mask_topk_filtered" : "mask_topk");
     if (nc > 1) {
         launch_pdl(topk_merge_kernel, ceil_div(n_rows, kTopkWarps), kTopkWarps * 32, 0, (cudaStream_t)stream, (const float*)cv,
                    (const int32_t*)ci, n_rows, 1, nc * K, (int64_t)0, K, out_val, out_idx);
         HVAE_LAUNCH_CHECK("mask_topk merge");
     }
     return 0;
+}
+
+// scratch cand_val / cand_idx: [n_rows, hvae_mask_topk_chunks(n_rows, N) * K] (may be NULL when that is 1)
+int hvae_mask_topk(float* S, int64_t lds, int n_rows, int N, int item_offset, const int64_t* indptr, const int32_t* indices,
+                   const int32_t* rows, int exclude_seen, int K, float* cand_val, int32_t* cand_idx, float* out_val, int32_t* out_idx,
+                   void* stream) {
+    return mask_topk(S, lds, n_rows, N, item_offset, indptr, indices, rows, exclude_seen, nullptr, 0, nullptr, K, cand_val, cand_idx,
+                     out_val, out_idx, stream);
+}
+
+// The same restricted to per-row allow-sets (bitmaps over global item ids, see hvae_tc_score_topk_filtered); allow == NULL is
+// hvae_mask_topk.  Slots a row cannot fill hold (-inf, -1).
+int hvae_mask_topk_filtered(float* S, int64_t lds, int n_rows, int N, int item_offset, const int64_t* indptr, const int32_t* indices,
+                            const int32_t* rows, int exclude_seen, const uint32_t* allow, int64_t allow_stride_words,
+                            const int32_t* allow_of_row, int K, float* cand_val, int32_t* cand_idx, float* out_val, int32_t* out_idx,
+                            void* stream) {
+    if (allow) {
+        HVAE_REQUIRE(allow_of_row, "mask_topk_filtered: allow needs allow_of_row");
+        HVAE_REQUIRE(item_offset >= 0 && allow_stride_words >= ((int64_t)item_offset + N + 31) / 32,
+                     "mask_topk_filtered: allow_stride_words=%lld does not cover items up to %lld", (long long)allow_stride_words,
+                     (long long)item_offset + N);
+    }
+    return mask_topk(S, lds, n_rows, N, item_offset, indptr, indices, rows, exclude_seen, allow, allow_stride_words, allow_of_row, K,
+                     cand_val, cand_idx, out_val, out_idx, stream);
 }
 
 int hvae_topk_merge(const float* cval, const int32_t* cidx, int n_rows, int GK, int K, float* out_val, int32_t* out_idx, void* stream) {

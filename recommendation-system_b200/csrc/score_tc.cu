@@ -44,6 +44,10 @@ struct StatsParams {
     const int64_t* indptr;   // seen items (CSR over users), may be null
     const int32_t* indices;
     const int32_t* rows;     // user ids of the batch rows (null = identity)
+    // TOPK with FILTER: item allow-sets, bit i of a bitmap row = global item i may be returned
+    const uint32_t* allow;        // [F, allow_stride] words
+    int64_t allow_stride;
+    const int32_t* allow_of_row;  // [B] bitmap row of each batch row, -1 = unrestricted
 };
 
 // One-pass mode (hvae_tc_score_onepass): softmax numerators are taken against a per-row shift c_b that does not depend on the
@@ -75,8 +79,28 @@ __device__ __forceinline__ float topk_key_value(uint64_t k) {
 
 __device__ __forceinline__ bool better(float v, int i, float tv, int ti) { return v > tv || (v == tv && i > ti); }
 
+// The allow bits of the 256 items g0.. of one tile as eight words (bit j of aw[c] = item g0 + 32c + j), from the row's bitmap
+// (null = everything allowed).  g0 need not be a multiple of 32: each word is funnel-shifted out of two neighbours.  Words past
+// the one holding item g_end - 1 are not read (the epilogue drops those columns anyway).
+__device__ __forceinline__ void tile_allow_words(const uint32_t* arow, int g0, int g_end, uint32_t (&aw)[8]) {
+    if (!arow) {
+#pragma unroll
+        for (int e = 0; e < 8; ++e) aw[e] = 0xFFFFFFFFu;
+        return;
+    }
+    const int w0 = g0 >> 5, sh = g0 & 31, wlast = (g_end - 1) >> 5;
+    uint32_t raw[9];
+#pragma unroll
+    for (int e = 0; e < 8; ++e) raw[e] = w0 + e <= wlast ? __ldg(arow + w0 + e) : 0u;
+    raw[8] = sh && w0 + 8 <= wlast ? __ldg(arow + w0 + 8) : 0u;
+#pragma unroll
+    for (int e = 0; e < 8; ++e) aw[e] = __funnelshift_r(raw[e], raw[e + 1], sh);
+}
+
 // STG = operand ring depth; KREG > 0: top-K list of KREG >= K sorted keys per row in registers, KREG == 0: list in shared memory.
-template <int MODE, int STG, int KREG>
+// FILTER (TOPK only): a column is a candidate only if the row's allow bitmap has its bit; the words are ANDed into the
+// compare mask of each 32-column chunk, so a rejected column never reaches the insertion loop.
+template <int MODE, int STG, int KREG, bool FILTER = false>
 __global__ void __launch_bounds__(192, 1) score_stats_kernel(const __grid_constant__ CUtensorMap tmU,
                                                              const __grid_constant__ CUtensorMap tmE, StatsParams P) {
     constexpr int STAGES = STG;      // (shadows the file-level default)
@@ -178,8 +202,15 @@ __global__ void __launch_bounds__(192, 1) score_stats_kernel(const __grid_consta
                 next_seen = seen_p < seen_e ? P.indices[seen_p] : INT_MAX;
             }
         }
+        const uint32_t* arow = nullptr;
+        if constexpr (FILTER) {
+            const int f = row_ok ? P.allow_of_row[row] : -1;
+            if (f >= 0) arow = P.allow + (size_t)f * P.allow_stride;
+        }
         for (int t = t0, ti = 0; t < t1; ++t, ++ti) {
             const int acc = ti & 1;
+            uint32_t aw[8];
+            if constexpr (FILTER) tile_allow_words(arow, P.item_offset + t * BN, P.item_offset + P.N, aw);   // in flight during the MMA
             mbar_wait(&bars->tmem_full[acc], (ti >> 1) & 1);
             tc_fence_after();
             const int col0 = t * BN;
@@ -226,6 +257,12 @@ __global__ void __launch_bounds__(192, 1) score_stats_kernel(const __grid_consta
                     for (int j = 0; j < 32; ++j) mbits |= (v[j] >= thr_v) ? (1u << j) : 0u;
                     const int left = n_valid - c * 32;
                     if (left < 32) mbits &= (1u << left) - 1u;
+                    if constexpr (FILTER) {
+                        uint32_t a = aw[0];
+#pragma unroll
+                        for (int e = 1; e < 8; ++e) a = (e == c) ? aw[e] : a;
+                        mbits &= a;
+                    }
                     if (!row_ok) mbits = 0;
                     while (mbits) {
                         const int j = __ffs(mbits) - 1;
@@ -949,6 +986,43 @@ static int pick_topk_splits(int m_tiles, int n_tiles) {
 constexpr size_t kStatsSmem = STAGES * STAGE_BYTES + 256 + 1024;                                        // LSE, register-list top-K
 constexpr size_t kStatsSmemList = STAGES_SMEM_LIST * STAGE_BYTES + 256 + BM * (MAXK_TC + 1) * 8 + 1024;   // shared-memory-list top-K
 
+// Sets the shared-memory limit of every top-K list bucket of one FILTER flavour (once per process).
+template <bool FILTER>
+static int topk_set_attrs() {
+    static bool attr_set = false;
+    if (!attr_set) {
+        HVAE_CUDA(cudaFuncSetAttribute(score_stats_kernel<MODE_TOPK, STAGES, 8, FILTER>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kStatsSmem));
+        HVAE_CUDA(cudaFuncSetAttribute(score_stats_kernel<MODE_TOPK, STAGES, 12, FILTER>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kStatsSmem));
+        HVAE_CUDA(cudaFuncSetAttribute(score_stats_kernel<MODE_TOPK, STAGES, 16, FILTER>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kStatsSmem));
+        HVAE_CUDA(cudaFuncSetAttribute(score_stats_kernel<MODE_TOPK, STAGES, 20, FILTER>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kStatsSmem));
+        HVAE_CUDA(cudaFuncSetAttribute(score_stats_kernel<MODE_TOPK, STAGES, 24, FILTER>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kStatsSmem));
+        HVAE_CUDA(cudaFuncSetAttribute(score_stats_kernel<MODE_TOPK, STAGES, 32, FILTER>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kStatsSmem));
+        HVAE_CUDA(cudaFuncSetAttribute(score_stats_kernel<MODE_TOPK, STAGES_SMEM_LIST, 0, FILTER>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                       (int)kStatsSmemList));
+        attr_set = true;
+    }
+    return 0;
+}
+
+// the list capacity is a compile-time size (register arrays): the smallest bucket that holds K.  A list longer than K costs twice: the
+// admission threshold is its LAST entry (more insertions) and every insertion walks the whole list -- hence buckets at the evaluation
+// protocol's own K values (5, 10, 20: src/ml/evaluate.py k_values)
+template <bool FILTER>
+static int launch_topk(int K, dim3 grid, cudaStream_t st, const CUtensorMap& tmU, const CUtensorMap& tmE, const StatsParams& P) {
+    if (int rc = topk_set_attrs<FILTER>()) return rc;
+    static const int force_kreg = getenv("HVAE_TOPK_KREG") ? atoi(getenv("HVAE_TOPK_KREG")) : 0;        // A/B runs: a larger bucket than needed
+    if (force_kreg >= K && force_kreg <= MAXK_REG) K = force_kreg;       // (P.K, the number of results written, stays)
+    if (K <= 8) launch_pdl(score_stats_kernel<MODE_TOPK, STAGES, 8, FILTER>, grid, 192, kStatsSmem, st, tmU, tmE, P);
+    else if (K <= 12) launch_pdl(score_stats_kernel<MODE_TOPK, STAGES, 12, FILTER>, grid, 192, kStatsSmem, st, tmU, tmE, P);
+    else if (K <= 16) launch_pdl(score_stats_kernel<MODE_TOPK, STAGES, 16, FILTER>, grid, 192, kStatsSmem, st, tmU, tmE, P);
+    else if (K <= 20) launch_pdl(score_stats_kernel<MODE_TOPK, STAGES, 20, FILTER>, grid, 192, kStatsSmem, st, tmU, tmE, P);
+    else if (K <= 24) launch_pdl(score_stats_kernel<MODE_TOPK, STAGES, 24, FILTER>, grid, 192, kStatsSmem, st, tmU, tmE, P);
+    else if (K <= MAXK_REG) launch_pdl(score_stats_kernel<MODE_TOPK, STAGES, 32, FILTER>, grid, 192, kStatsSmem, st, tmU, tmE, P);
+    else launch_pdl(score_stats_kernel<MODE_TOPK, STAGES_SMEM_LIST, 0, FILTER>, grid, 192, kStatsSmemList, st, tmU, tmE, P);
+    HVAE_LAUNCH_CHECK(FILTER ? "tc_score_topk_filtered" : "tc_score_topk");
+    return 0;
+}
+
 }  // namespace tc
 }  // namespace hvae
 
@@ -1081,10 +1155,9 @@ int hvae_tc_score_lse_grad(const void* U, int ldu, int B, const void* E, int lde
     return launch_grad(U, ldu, B, E, lde, N, d, nullptr, workspace, workspace + (size_t)B * ns, ns, lse, Opart, ldo, (cudaStream_t)stream);
 }
 
-// Top-K over the N items of E (global ids item_offset..item_offset+N).  cand_val / cand_idx: [B, n_splits*K] scratch;
-// the caller reduces them with hvae_topk_merge.  K <= 128 (K <= 32: register-resident lists; above: shared-memory lists).
-int hvae_tc_score_topk(const void* U, int ldu, int B, const void* E, int lde, int N, int d, int item_offset, const int64_t* indptr,
-                       const int32_t* indices, const int32_t* rows, int K, float* cand_val, int32_t* cand_idx, void* stream) {
+static int score_topk(const void* U, int ldu, int B, const void* E, int lde, int N, int d, int item_offset, const int64_t* indptr,
+                      const int32_t* indices, const int32_t* rows, const uint32_t* allow, int64_t allow_stride,
+                      const int32_t* allow_of_row, int K, float* cand_val, int32_t* cand_idx, void* stream) {
     if (B == 0) return 0;
     HVAE_REQUIRE(K >= 1 && K <= MAXK_TC, "tc_score_topk: K=%d outside [1,%d]", K, MAXK_TC);
     CUtensorMap tmU, tmE;
@@ -1097,36 +1170,35 @@ int hvae_tc_score_topk(const void* U, int ldu, int B, const void* E, int lde, in
     P.tiles_per_split = ceil_div(n_tiles, P.n_splits);
     P.cand_val = cand_val; P.cand_idx = cand_idx;
     P.indptr = indptr; P.indices = indices; P.rows = rows;
-    static bool attr_set = false;
-    if (!attr_set) {
-        HVAE_CUDA(cudaFuncSetAttribute(score_stats_kernel<MODE_TOPK, STAGES, 8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kStatsSmem));
-        HVAE_CUDA(cudaFuncSetAttribute(score_stats_kernel<MODE_TOPK, STAGES, 12>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kStatsSmem));
-        HVAE_CUDA(cudaFuncSetAttribute(score_stats_kernel<MODE_TOPK, STAGES, 16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kStatsSmem));
-        HVAE_CUDA(cudaFuncSetAttribute(score_stats_kernel<MODE_TOPK, STAGES, 20>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kStatsSmem));
-        HVAE_CUDA(cudaFuncSetAttribute(score_stats_kernel<MODE_TOPK, STAGES, 24>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kStatsSmem));
-        HVAE_CUDA(cudaFuncSetAttribute(score_stats_kernel<MODE_TOPK, STAGES, 32>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kStatsSmem));
-        HVAE_CUDA(cudaFuncSetAttribute(score_stats_kernel<MODE_TOPK, STAGES_SMEM_LIST, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                       (int)kStatsSmemList));
-        attr_set = true;
-    }
+    P.allow = allow; P.allow_stride = allow_stride; P.allow_of_row = allow_of_row;
     const dim3 grid(m_tiles, P.n_splits);
-    cudaStream_t st = (cudaStream_t)stream;
-    // the list capacity is a compile-time size (register arrays): the smallest bucket that holds K.  A list longer than K costs twice: the
-    // admission threshold is its LAST entry (more insertions) and every insertion walks the whole list -- hence buckets at the evaluation
-    // protocol's own K values (5, 10, 20: src/ml/evaluate.py k_values)
-    static const int force_kreg = getenv("HVAE_TOPK_KREG") ? atoi(getenv("HVAE_TOPK_KREG")) : 0;        // A/B runs: a larger bucket than needed
-    if (force_kreg >= K && force_kreg <= MAXK_REG) K = force_kreg;       // (P.K, the number of results written, stays)
-    if (K <= 8) launch_pdl(score_stats_kernel<MODE_TOPK, STAGES, 8>, grid, 192, kStatsSmem, st, tmU, tmE, P);
-    else if (K <= 12) launch_pdl(score_stats_kernel<MODE_TOPK, STAGES, 12>, grid, 192, kStatsSmem, st, tmU, tmE, P);
-    else if (K <= 16) launch_pdl(score_stats_kernel<MODE_TOPK, STAGES, 16>, grid, 192, kStatsSmem, st, tmU, tmE, P);
-    else if (K <= 20) launch_pdl(score_stats_kernel<MODE_TOPK, STAGES, 20>, grid, 192, kStatsSmem, st, tmU, tmE, P);
-    else if (K <= 24) launch_pdl(score_stats_kernel<MODE_TOPK, STAGES, 24>, grid, 192, kStatsSmem, st, tmU, tmE, P);
-    else if (K <= MAXK_REG) launch_pdl(score_stats_kernel<MODE_TOPK, STAGES, 32>, grid, 192, kStatsSmem, st, tmU, tmE, P);
-    else launch_pdl(score_stats_kernel<MODE_TOPK, STAGES_SMEM_LIST, 0>, grid, 192, kStatsSmemList, st, tmU, tmE, P);
-    HVAE_LAUNCH_CHECK("tc_score_topk");
-    return 0;
+    if (allow) return launch_topk<true>(K, grid, (cudaStream_t)stream, tmU, tmE, P);
+    return launch_topk<false>(K, grid, (cudaStream_t)stream, tmU, tmE, P);
 }
 
+// Top-K over the N items of E (global ids item_offset..item_offset+N).  cand_val / cand_idx: [B, n_splits*K] scratch;
+// the caller reduces them with hvae_topk_merge.  K <= 128 (K <= 32: register-resident lists; above: shared-memory lists).
+int hvae_tc_score_topk(const void* U, int ldu, int B, const void* E, int lde, int N, int d, int item_offset, const int64_t* indptr,
+                       const int32_t* indices, const int32_t* rows, int K, float* cand_val, int32_t* cand_idx, void* stream) {
+    return score_topk(U, ldu, B, E, lde, N, d, item_offset, indptr, indices, rows, nullptr, 0, nullptr, K, cand_val, cand_idx, stream);
+}
+
+// The same restricted to per-row allow-sets: row b may only return items whose bit is set in allow[allow_of_row[b]] (bitmaps over
+// global item ids, allow_stride_words >= ceil((item_offset + N) / 32)); allow_of_row[b] == -1: unrestricted.  allow == NULL is
+// hvae_tc_score_topk.  A row with fewer than K admissible items pads its list with (-inf, -1).
+int hvae_tc_score_topk_filtered(const void* U, int ldu, int B, const void* E, int lde, int N, int d, int item_offset,
+                                const int64_t* indptr, const int32_t* indices, const int32_t* rows, const uint32_t* allow,
+                                int64_t allow_stride_words, const int32_t* allow_of_row, int K, float* cand_val, int32_t* cand_idx,
+                                void* stream) {
+    if (allow) {
+        HVAE_REQUIRE(allow_of_row, "tc_score_topk_filtered: allow needs allow_of_row");
+        HVAE_REQUIRE(item_offset >= 0 && allow_stride_words >= ((int64_t)item_offset + N + 31) / 32,
+                     "tc_score_topk_filtered: allow_stride_words=%lld does not cover items up to %lld", (long long)allow_stride_words,
+                     (long long)item_offset + N);
+    }
+    return score_topk(U, ldu, B, E, lde, N, d, item_offset, indptr, indices, rows, allow, allow_stride_words, allow_of_row, K,
+                      cand_val, cand_idx, stream);
+}
 
 // 1 or 2 numerator sums per (split, row): the pair kernel's two CTAs each report the tiles they owned
 size_t hvae_tc_onepass_subparts(int d) { return grad_kind(d) != GRAD_SINGLE ? 2 : 1; }

@@ -697,8 +697,12 @@ class Engine:
         ml = self.encode(batch, None)
         return self.latent_and_project(batch.B, ml, None, None, want_kl=False)
 
-    def topk(self, batch: Batch, K: int, exclude_seen=True, item_lo=0, item_hi=None):
-        """Full ranking: scores over items [item_lo,item_hi) -> mask seen -> top-K (value, global index)."""
+    def topk(self, batch: Batch, K: int, exclude_seen=True, item_lo=0, item_hi=None, *, mask=None, allow=None):
+        """Full ranking: scores over items [item_lo,item_hi) -> mask seen -> top-K (value, global index).
+
+        mask = (indptr int64 [B+1], indices int32): sorted items to leave out per batch row, used instead of the seen rows
+        (exclude_seen is then not looked at).  allow = (bitmaps int32 [F, words], allow_of_row int32 [B]): item allow-sets
+        over global ids, -1 = unrestricted.  Slots a filtered row cannot fill hold (-inf, -1)."""
         lay, ws, lib, st = self.lay, self.ws, self.lib, self.stream
         item_hi = lay.N if item_hi is None else item_hi
         n_it = item_hi - item_lo
@@ -708,7 +712,7 @@ class Engine:
         out_idx = torch.empty(B, K, dtype=torch.int32, device=self.dev)
         if self.precision != "fp32":
             from . import tc
-            if tc.topk_bf16(self, batch, u, K, exclude_seen, item_lo, item_hi, out_val, out_idx):
+            if tc.topk_bf16(self, batch, u, K, exclude_seen, item_lo, item_hi, out_val, out_idx, mask, allow):
                 return out_val, out_idx
         csr = batch.csr
         bc = max(1, min(B, (256 * 1024 * 1024) // max(1, n_it)))
@@ -721,6 +725,17 @@ class Engine:
             nc = int(lib.mask_topk_chunks(nb, n_it))
             cv = ws.get("topk_cand_v", (nb, nc * K))
             ci = ws.get("topk_cand_i", (nb, nc * K), torch.int32)
-            lib.mask_topk(p(S), n_it, nb, n_it, item_lo, p(csr.indptr), p(csr.indices), rows_ptr, 1 if exclude_seen else 0, K,
-                          p(cv), p(ci), out_val.data_ptr() + 4 * r0 * K, out_idx.data_ptr() + 4 * r0 * K, st)
+            ov, oi = out_val.data_ptr() + 4 * r0 * K, out_idx.data_ptr() + 4 * r0 * K
+            if mask is None and allow is None:
+                lib.mask_topk(p(S), n_it, nb, n_it, item_lo, p(csr.indptr), p(csr.indices), rows_ptr, 1 if exclude_seen else 0, K,
+                              p(cv), p(ci), ov, oi, st)
+                continue
+            if mask is not None:        # rows of the mask CSR are batch rows: start at row r0 of it
+                indptr_ptr, indices_ptr, rows_ptr, excl = mask[0].data_ptr() + 8 * r0, p(mask[1]), None, 1
+            else:
+                indptr_ptr, indices_ptr, excl = p(csr.indptr), p(csr.indices), 1 if exclude_seen else 0
+            bm, aor = allow if allow is not None else (None, None)
+            lib.mask_topk_filtered(p(S), n_it, nb, n_it, item_lo, indptr_ptr, indices_ptr, rows_ptr, excl, p(bm),
+                                   0 if bm is None else bm.stride(0), None if aor is None else aor.data_ptr() + 4 * r0, K,
+                                   p(cv), p(ci), ov, oi, st)
         return out_val, out_idx

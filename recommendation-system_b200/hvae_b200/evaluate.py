@@ -10,6 +10,7 @@ argsort()[::-1] gives; the reference's default argsort is unstable, so its order
 from __future__ import annotations
 
 import logging
+import threading
 from pathlib import Path
 
 import numpy as np
@@ -75,11 +76,74 @@ class RecommendationEvaluator:
         self.n_items = interaction_matrix.n_items if isinstance(interaction_matrix, DeviceCSR) else interaction_matrix.shape[1]
         self.batch_users = batch_users
         self._csr = interaction_matrix if isinstance(interaction_matrix, DeviceCSR) else DeviceCSR.from_scipy(interaction_matrix, device)
+        # (int32 [F, ceil(n_items / 32)] item bitmaps of the named filters, name -> row): replaced as a whole, never written in
+        # place, so a top-K call that took the pair keeps a consistent table while another thread registers a filter
+        self._filters: tuple = (None, {})
+        self._filters_lock = threading.Lock()
+
+    # -- item filters ------------------------------------------------------------------------------------------------
+    def add_item_filter(self, name: str, item_indices) -> None:
+        """Registers (or replaces) the allow-set `name`: topk_users(..., item_filter=name) then only returns these items."""
+        idx = np.asarray(item_indices, dtype=np.int64).reshape(-1)
+        if idx.size and (idx.min() < 0 or idx.max() >= self.n_items):
+            raise ValueError(f"item filter {name!r}: item indices must lie in [0, {self.n_items})")
+        words = (self.n_items + 31) // 32
+        bits = np.zeros(words * 32, dtype=bool)
+        bits[idx] = True
+        row = torch.as_tensor(np.packbits(bits, bitorder="little").view(np.int32), device=self.device)   # bit i of word w: item 32w + i
+        with self._filters_lock:
+            table, rows = self._filters
+            if name in rows:
+                table = table.clone()
+                table[rows[name]] = row
+            else:
+                rows = {**rows, name: 0 if table is None else table.shape[0]}
+                table = row[None] if table is None else torch.cat([table, row[None]])
+            self._filters = (table, rows)
+
+    @staticmethod
+    def _allow_of_row(item_filter, n, filter_row):
+        """-> int32 [n] bitmap rows (-1 = unrestricted) on the host, or None when no user is restricted."""
+        names = [item_filter] * n if item_filter is None or isinstance(item_filter, str) else list(item_filter)
+        if len(names) != n:
+            raise ValueError(f"item_filter: {len(names)} entries for {n} users")
+        if all(nm is None for nm in names):
+            return None
+        for nm in names:
+            if nm is not None and (not isinstance(nm, str) or nm not in filter_row):
+                raise ValueError(f"unknown item filter {nm!r}")
+        return np.array([-1 if nm is None else filter_row[nm] for nm in names], dtype=np.int32)
+
+    def _mask_csr(self, rows, excl, exclude_seen):
+        """Sorted union per batch row of the user's seen items (exclude_seen) and the row's exclusion list, built on the device:
+        -> (indptr int64 [n+1], indices int32)."""
+        n, N, dev = rows.shape[0], self.n_items, self.device
+        keys = []
+        if exclude_seen:
+            start, end = self._csr.indptr[rows.long()], self._csr.indptr[rows.long() + 1]
+            cnt = end - start
+            row_of = torch.repeat_interleave(torch.arange(n, device=dev), cnt)
+            pos = torch.arange(int(cnt.sum()), device=dev) - torch.repeat_interleave(torch.cumsum(cnt, 0) - cnt, cnt)
+            keys.append(row_of * N + self._csr.indices[start[row_of] + pos].long())
+        lens = [len(e) for e in excl]
+        if sum(lens):
+            ex = torch.as_tensor(np.concatenate([np.asarray(e, dtype=np.int64).reshape(-1) for e in excl]), device=dev)
+            keys.append(torch.repeat_interleave(torch.arange(n, device=dev), torch.as_tensor(lens, device=dev)) * N + ex)
+        key = torch.unique(torch.cat(keys)) if keys else torch.empty(0, dtype=torch.int64, device=dev)   # sorted
+        indptr = torch.zeros(n + 1, dtype=torch.int64, device=dev)
+        indptr[1:] = torch.cumsum(torch.bincount(key // N, minlength=n), 0)
+        return indptr, (key % N).to(torch.int32)
 
     # -- batched primitives ----------------------------------------------------------------------------------------
-    def topk_users(self, user_indices, top_k: int, exclude_seen: bool = True):
-        """(values [n,K] f32, indices [n,K] int32) device tensors for the given users."""
+    def topk_users(self, user_indices, top_k: int, exclude_seen: bool = True, *, item_filter=None, exclude=None):
+        """(values [n,K] f32, indices [n,K] int32) device tensors for the given users.
+
+        item_filter: the name of a filter registered with add_item_filter, or one name (or None) per user: that user only gets
+        items of the filter.  exclude: one array of item indices per user, left out on top of the seen items.  A user with
+        fewer than K admissible items gets (-inf, -1) in the remaining slots."""
         users = torch.as_tensor(np.asarray(user_indices, dtype=np.int32), device=self.device)
+        if item_filter is not None or exclude is not None:
+            return self._topk_filtered(users, top_k, exclude_seen, item_filter, exclude)
         eng = self.model.engine
         from . import tc
         if eng.precision != "fp32" and exclude_seen and top_k <= tc.MAX_K_REG and users.shape[0] >= 2 * self.batch_users:
@@ -98,6 +162,34 @@ class RecommendationEvaluator:
             for s in range(0, users.shape[0], self.batch_users):
                 rows = users[s:s + self.batch_users].contiguous()
                 v, i = eng.topk(Batch(self._csr, rows, rows.shape[0], 1), top_k, exclude_seen)
+                vals.append(v)
+                idxs.append(i)
+        if not vals:
+            return (torch.empty(0, top_k, device=self.device), torch.empty(0, top_k, dtype=torch.int32, device=self.device))
+        return torch.cat(vals), torch.cat(idxs)
+
+    def _topk_filtered(self, users, top_k, exclude_seen, item_filter, exclude):
+        n = users.shape[0]
+        with self._filters_lock:
+            table, filter_row = self._filters
+        aor = self._allow_of_row(item_filter, n, filter_row)
+        if exclude is not None:
+            exclude = list(exclude)
+            if len(exclude) != n:
+                raise ValueError(f"exclude: {len(exclude)} lists for {n} users")
+            for e in exclude:
+                e = np.asarray(e).reshape(-1)
+                if e.size and (e.min() < 0 or e.max() >= self.n_items):
+                    raise ValueError(f"exclude: item indices must lie in [0, {self.n_items})")
+        aor_d = None if aor is None else torch.as_tensor(aor, device=self.device)
+        eng = self.model.engine
+        vals, idxs = [], []
+        with torch.no_grad():
+            for s in range(0, n, self.batch_users):
+                rows = users[s:s + self.batch_users].contiguous()
+                mask = None if exclude is None else self._mask_csr(rows, exclude[s:s + rows.shape[0]], exclude_seen)
+                allow = None if aor_d is None else (table, aor_d[s:s + rows.shape[0]].contiguous())
+                v, i = eng.topk(Batch(self._csr, rows, rows.shape[0], 1), top_k, exclude_seen, mask=mask, allow=allow)
                 vals.append(v)
                 idxs.append(i)
         if not vals:

@@ -74,15 +74,20 @@ def score_loss_bf16(eng, batch, u, want_grad):
     return lse, dot, xsum, O, xsum
 
 
-def topk_bf16(eng, batch, u, K, exclude_seen, item_lo, item_hi, out_val, out_idx) -> bool:
+def topk_bf16(eng, batch, u, K, exclude_seen, item_lo, item_hi, out_val, out_idx, mask=None, allow=None) -> bool:
     """Fused score + seen-mask + top-K over items [item_lo, item_hi).  False if K is beyond the fused kernel."""
     if K > MAX_K_TC:
         return False
-    return topk_bf16_from_ub(eng, batch, user_vectors_bf16(eng, u, batch.B), K, exclude_seen, item_lo, item_hi, out_val, out_idx)
+    return topk_bf16_from_ub(eng, batch, user_vectors_bf16(eng, u, batch.B), K, exclude_seen, item_lo, item_hi, out_val, out_idx,
+                             mask, allow)
 
 
-def topk_bf16_from_ub(eng, batch, ub, K, exclude_seen, item_lo, item_hi, out_val, out_idx) -> bool:
-    """The same with the bf16 user vectors [B, r8(d)] already at hand (item-sharded evaluation all-gathers them)."""
+def topk_bf16_from_ub(eng, batch, ub, K, exclude_seen, item_lo, item_hi, out_val, out_idx, mask=None, allow=None) -> bool:
+    """The same with the bf16 user vectors [B, r8(d)] already at hand (item-sharded evaluation all-gathers them).
+
+    mask = (indptr int64 [B+1], indices int32): items to leave out, one sorted row per BATCH row; it replaces the batch's
+    seen rows (exclude_seen is then not looked at).  allow = (bitmaps int32 [F, words], allow_of_row int32 [B]): row b only
+    returns items whose bit is set in bitmaps[allow_of_row[b]] (-1: unrestricted); slots it cannot fill hold (-inf, -1)."""
     if K > MAX_K_TC:
         return False
     lay, ws, lib, st = eng.lay, eng.ws, eng.lib, eng.stream
@@ -95,7 +100,16 @@ def topk_bf16_from_ub(eng, batch, ub, K, exclude_seen, item_lo, item_hi, out_val
     ci = ws.get("tc_cand_i", (B, ns * K), torch.int32)
     csr = batch.csr
     with eng.span("score_topk"):
-        lib.tc_score_topk(p(ub), ld8, B, Eb.data_ptr() + 2 * item_lo * ld8, ld8, n_it, d, item_lo,
-                          p(csr.indptr) if exclude_seen else None, p(csr.indices), p(batch.rows), K, p(cv), p(ci), st)
+        if mask is None and allow is None:
+            lib.tc_score_topk(p(ub), ld8, B, Eb.data_ptr() + 2 * item_lo * ld8, ld8, n_it, d, item_lo,
+                              p(csr.indptr) if exclude_seen else None, p(csr.indices), p(batch.rows), K, p(cv), p(ci), st)
+        else:
+            if mask is not None:
+                indptr, indices, rows = mask[0], mask[1], None
+            else:
+                indptr, indices, rows = (csr.indptr if exclude_seen else None), csr.indices, batch.rows
+            bm, aor = allow if allow is not None else (None, None)
+            lib.tc_score_topk_filtered(p(ub), ld8, B, Eb.data_ptr() + 2 * item_lo * ld8, ld8, n_it, d, item_lo, p(indptr), p(indices),
+                                       p(rows), p(bm), 0 if bm is None else bm.stride(0), p(aor), K, p(cv), p(ci), st)
     lib.topk_merge(p(cv), p(ci), B, ns * K, K, p(out_val), p(out_idx), st)
     return True
