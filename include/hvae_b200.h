@@ -184,6 +184,13 @@ int hvae_mask_topk_filtered(float* S, int64_t lds, int n_rows, int N, int item_o
                             const int32_t* indices, const int32_t* rows, int exclude_seen, const uint32_t* allow,
                             int64_t allow_stride_words, const int32_t* allow_of_row, int K, float* cand_val, int32_t* cand_idx,
                             float* out_val, int32_t* out_idx, void* stream);
+/* The same, sampling: out_val / out_idx are a K-item Gumbel-top-K draw per row (see hvae_tc_score_topk_sampled).  out_val
+ * holds the rows' keys, not their scores; allow == NULL: unrestricted. */
+int hvae_mask_topk_sampled(float* S, int64_t lds, int n_rows, int N, int item_offset, const int64_t* indptr,
+                           const int32_t* indices, const int32_t* rows, int exclude_seen, const uint32_t* allow,
+                           int64_t allow_stride_words, const int32_t* allow_of_row, const float* row_inv_tau,
+                           const uint64_t* row_seed, int K, float* cand_val, int32_t* cand_idx, float* out_val,
+                           int32_t* out_idx, void* stream);
 int hvae_topk_merge(const float* cval, const int32_t* cidx, int n_rows, int GK, int K, float* out_val, int32_t* out_idx,
                     void* stream);
 /* The same merge over the blocks of an all-gather, read in place: rank g's K candidates of row r are at
@@ -191,7 +198,8 @@ int hvae_topk_merge(const float* cval, const int32_t* cidx, int n_rows, int GK, 
 int hvae_topk_merge_groups(const float* cval, const int32_t* cidx, int n_rows, int n_groups, int64_t group_stride, int K,
                            float* out_val, int32_t* out_idx, void* stream);
 /* Negative-sampling protocol (evaluate.py:149-185): scores of C candidates per row (candidate 0 = test item) and the
- * 0-based rank of candidate 0 under a stable descending sort.  cand: int32 [B, C]; scores may be NULL. */
+ * 0-based rank of candidate 0 under a stable descending sort.  cand: int32 [B, C]; scores may be NULL.  A candidate id
+ * of -1 (an empty top-K slot) scores -inf and reads nothing. */
 int hvae_candidate_rank(const void* U, int ldu, const void* E, int lde, int d, int is_bf16, const int32_t* cand, int C, int B,
                         float* scores, int32_t* rank, void* stream);
 /* Recall/NDCG/HR@K (evaluate.py:32-54,90-98) */
@@ -221,6 +229,20 @@ int hvae_tc_score_topk_filtered(const void* U, int ldu, int B, const void* E, in
                                 const int64_t* indptr, const int32_t* indices, const int32_t* rows,
                                 const uint32_t* allow, int64_t allow_stride_words, const int32_t* allow_of_row,
                                 int K, float* cand_val, int32_t* cand_idx, void* stream);
+/* The same, sampling (Gumbel-top-K): row b with row_inv_tau[b] = 1/tau != 0 ranks the keys
+ *     key_i = fmaf(s_bi, row_inv_tau[b], g_i),   g_i = -logf(-logf(u_i)),   u_i = ((r_i >> 9) + 0.5f) * 2^-23,
+ *     r_i = word (i & 3) of Philox4x32-10 with key {seed lo, seed hi} = row_seed[b], counter {i >> 2, 0, 0x53414D50, 0},
+ * i the GLOBAL item id, logf the accurate (not __logf) logarithm.  Its K best keys are a draw of K items without replacement
+ * from softmax(s_b / tau) over the admissible items (Plackett-Luce), and the first k of them a k-item draw: the noise depends
+ * on (row_seed[b], i) only, not on the batch row, the item split, the shard or K.  A row with row_inv_tau[b] == 0 gets what
+ * hvae_tc_score_topk_filtered gives.  Seen, excluded and disallowed items are never drawn; slots a row cannot fill hold
+ * (-inf, -1).  cand_val holds KEYS (merge them with hvae_topk_merge); the caller recomputes the chosen items' scores
+ * (hvae_candidate_rank).  allow == NULL: unrestricted.  tau is meant to lie in [1e-3, 1e3]. */
+int hvae_tc_score_topk_sampled(const void* U, int ldu, int B, const void* E, int lde, int N, int d, int item_offset,
+                               const int64_t* indptr, const int32_t* indices, const int32_t* rows,
+                               const uint32_t* allow, int64_t allow_stride_words, const int32_t* allow_of_row,
+                               const float* row_inv_tau, const uint64_t* row_seed, int K, float* cand_val,
+                               int32_t* cand_idx, void* stream);
 
 /* Backward through the scores: O[b,:] = sum_i softmax(S_b)_i E_i with S recomputed on the tensor cores
  * (autograd of model.py:198,281; E is a frozen buffer, no dE).  lse from hvae_tc_score_lse.

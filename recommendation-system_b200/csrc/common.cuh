@@ -73,6 +73,37 @@ __device__ __forceinline__ float gelu_grad(float x) {
     return cdf + x * pdf;
 }
 
+// ---- counter-based random numbers (Philox4x32-10): counter {ctr_lo, ctr_hi, stream_id, 0}, key {seed_lo, seed_hi} ----
+__device__ __forceinline__ void philox_round(uint32_t (&c)[4], uint32_t k0, uint32_t k1) {
+    const uint64_t p0 = (uint64_t)0xD2511F53u * c[0], p1 = (uint64_t)0xCD9E8D57u * c[2];
+    const uint32_t n0 = (uint32_t)(p1 >> 32) ^ c[1] ^ k0, n2 = (uint32_t)(p0 >> 32) ^ c[3] ^ k1;
+    c[1] = (uint32_t)p1; c[3] = (uint32_t)p0; c[0] = n0; c[2] = n2;
+}
+__device__ __forceinline__ void philox(uint64_t seed, uint64_t ctr, uint32_t stream_id, uint32_t (&out)[4]) {
+    uint32_t c[4] = {(uint32_t)ctr, (uint32_t)(ctr >> 32), stream_id, 0u};
+    uint32_t k0 = (uint32_t)seed, k1 = (uint32_t)(seed >> 32);
+#pragma unroll
+    for (int r = 0; r < 10; ++r) { philox_round(c, k0, k1); k0 += 0x9E3779B9u; k1 += 0xBB67AE85u; }
+    out[0] = c[0]; out[1] = c[1]; out[2] = c[2]; out[3] = c[3];
+}
+
+// ---- Gumbel-top-K sampling of the top-K kernels (include/hvae_b200.h, hvae_tc_score_topk_sampled) ----
+// Item gi of a row with seed s draws word gi & 3 of philox(s, gi >> 2, kSampleStream): the noise depends on (seed, global
+// item id) only, never on the batch row, the item split, the shard or K.
+constexpr uint32_t kSampleStream = 0x53414D50u;   // "SAMP"
+// Above every Gumbel value gumbel_of() can return: the largest uniform, 1 - 2^-24, gives -log(-log(u)) = 16.63553 exactly, and
+// the two 1-ulp logf evaluations move that by less than 1e-5.  The top-K kernels admit a column only if
+// fmaf(s, inv_tau, kGumbelMax) >= threshold, which every key fmaf(s, inv_tau, g) at or above the threshold passes.
+constexpr float kGumbelMax = 16.64f;
+// u = ((r >> 9) + 0.5) 2^-23 is exact in fp32 and lies in [2^-24, 1 - 2^-24], so both logarithms are finite.
+__device__ __forceinline__ float gumbel_of(uint32_t r) {
+    const float u = ((float)(r >> 9) + 0.5f) * 1.1920928955078125e-7f;
+    return -logf(-logf(u));
+}
+__device__ __forceinline__ uint32_t pick4(const uint32_t (&w)[4], int k) {
+    return k == 0 ? w[0] : k == 1 ? w[1] : k == 2 ? w[2] : w[3];
+}
+
 __host__ __device__ __forceinline__ int ceil_div(int a, int b) { return (a + b - 1) / b; }
 __host__ __device__ __forceinline__ int round_up(int a, int b) { return (a + b - 1) / b * b; }
 

@@ -148,20 +148,7 @@ __global__ void __launch_bounds__(256) adam_touched_kernel(float4* __restrict__ 
     p[i] = pp; m[i] = mm; v[i] = vv;
 }
 
-// ---- counter-based noise (Philox4x32-10) for the throughput mode; parity mode passes torch's own tensors ----
-__device__ __forceinline__ void philox_round(uint32_t (&c)[4], uint32_t k0, uint32_t k1) {
-    const uint64_t p0 = (uint64_t)0xD2511F53u * c[0], p1 = (uint64_t)0xCD9E8D57u * c[2];
-    const uint32_t n0 = (uint32_t)(p1 >> 32) ^ c[1] ^ k0, n2 = (uint32_t)(p0 >> 32) ^ c[3] ^ k1;
-    c[1] = (uint32_t)p1; c[3] = (uint32_t)p0; c[0] = n0; c[2] = n2;
-}
-__device__ __forceinline__ void philox(uint64_t seed, uint64_t ctr, uint32_t stream_id, uint32_t (&out)[4]) {
-    uint32_t c[4] = {(uint32_t)ctr, (uint32_t)(ctr >> 32), stream_id, 0u};
-    uint32_t k0 = (uint32_t)seed, k1 = (uint32_t)(seed >> 32);
-#pragma unroll
-    for (int r = 0; r < 10; ++r) { philox_round(c, k0, k1); k0 += 0x9E3779B9u; k1 += 0xBB67AE85u; }
-    out[0] = c[0]; out[1] = c[1]; out[2] = c[2]; out[3] = c[3];
-}
-
+// ---- counter-based noise (philox, common.cuh) for the throughput mode; parity mode passes torch's own tensors ----
 __global__ void noise_mask_kernel(uint8_t* __restrict__ mask, int64_t n, float keep, uint64_t seed, uint64_t offset, uint32_t sid,
                                   const hvae_step_state* __restrict__ st) {
     pdl_prologue();

@@ -259,10 +259,14 @@ __global__ void __launch_bounds__(256) candidate_rank_kernel(const T* __restrict
     float s0 = 0.f;
     int r = 0;
     for (int c = 0; c < C; ++c) {
-        const T* e = E + (size_t)cand[(size_t)b * C + c] * lde;
-        float p = 0.f;
-        for (int k = lane; k < d; k += 32) p = fmaf(to_f(U[(size_t)b * ldu + k]), to_f(e[k]), p);
-        p = warp_sum(p);
+        const int ci = cand[(size_t)b * C + c];
+        float p = -INFINITY;            // id -1 (an empty top-K slot): no row of E is read
+        if (ci >= 0) {
+            const T* e = E + (size_t)ci * lde;
+            p = 0.f;
+            for (int k = lane; k < d; k += 32) p = fmaf(to_f(U[(size_t)b * ldu + k]), to_f(e[k]), p);
+            p = warp_sum(p);
+        }
         if (c == 0) s0 = p;
         else r += (p >= s0) ? 1 : 0;
         if (scores && lane == 0) scores[(size_t)b * C + c] = p;
@@ -365,14 +369,21 @@ constexpr int kTopkSeg = 8;          // 512-byte row segments per trip of the sc
 // FILTER: row r may only return items whose bit is set in allow[allow_of_row[r]] (-1: unrestricted).  The allow bits of a
 // trip's scores are fetched with the scores and applied when the trip is consumed (a disallowed score becomes -inf), so the
 // scan keeps its single read of S and its loads in flight; entries left at -inf are written with id -1.
-template <bool FILTER>
+// SAMPLE (with FILTER; allow may then be null): a row with row_inv_tau[r] != 0 ranks the Gumbel-top-K keys
+// fmaf(s, inv_tau, g), g the noise of (row_seed[r], global item id) (common.cuh: gumbel_of), and writes keys.  The trip and
+// segment tests take the bound fmaf(max, inv_tau, kGumbelMax) instead of the maximum, and only a lane whose segment passes
+// runs Philox (its 4 scores are one counter when the global id of the segment is a multiple of 4, else two) and the logs.
+// The probe is skipped for such rows.  A row with row_inv_tau[r] == 0 runs the FILTER kernel's arithmetic.
+template <bool FILTER, bool SAMPLE = false>
 __global__ void __launch_bounds__(kTopkWarps * 32) mask_topk_kernel(float* __restrict__ S, int64_t lds, int n_rows, int N,
                                                                     int item_offset, const int64_t* __restrict__ indptr,
                                                                     const int32_t* __restrict__ indices,
                                                                     const int32_t* __restrict__ rows, int exclude_seen, int K,
                                                                     int n_chunks, int chunk_len, float* __restrict__ out_val,
                                                                     int32_t* __restrict__ out_idx, const uint32_t* __restrict__ allow,
-                                                                    int64_t allow_stride, const int32_t* __restrict__ allow_of_row) {
+                                                                    int64_t allow_stride, const int32_t* __restrict__ allow_of_row,
+                                                                    const float* __restrict__ row_inv_tau,
+                                                                    const uint64_t* __restrict__ row_seed) {
     pdl_prologue();
     __shared__ float sv_all[kTopkWarps][kMaxK];
     __shared__ int si_all[kTopkWarps][kMaxK];
@@ -401,9 +412,33 @@ __global__ void __launch_bounds__(kTopkWarps * 32) mask_topk_kernel(float* __res
     auto fetch = [&](int base) { const int c = base + lane * 4; return (base < c1v && c < c1v) ? *reinterpret_cast<const float4*>(row + c) : ninf; };
     const uint32_t* arow = nullptr;
     if constexpr (FILTER) {
-        const int f = allow_of_row[r];
+        const int f = !SAMPLE || allow ? allow_of_row[r] : -1;
         if (f >= 0) arow = allow + (size_t)f * allow_stride;
     }
+    float s_a = 1.f, s_b = 0.f;     // SAMPLE: candidate bound fmaf(v, s_a, s_b)
+    uint64_t seed = 0;
+    if constexpr (SAMPLE) {
+        if (row_inv_tau[r] != 0.f) { s_a = row_inv_tau[r]; s_b = kGumbelMax; seed = row_seed[r]; }
+    }
+    const bool sampled = SAMPLE && s_b != 0.f;
+    auto bound = [&](float x) { if constexpr (SAMPLE) return fmaf(x, s_a, s_b); else return x; };
+    auto key1 = [&](float x, int g) {
+        uint32_t w[4];
+        philox(seed, (uint32_t)g >> 2, kSampleStream, w);
+        return fmaf(x, s_a, gumbel_of(pick4(w, g & 3)));
+    };
+    auto key4 = [&](float4 v, int g) {     // the 4 items g..g+3
+        uint32_t w[4], w2[4] = {0u, 0u, 0u, 0u};
+        const int sh = g & 3;
+        philox(seed, (uint32_t)g >> 2, kSampleStream, w);
+        if (sh) philox(seed, ((uint32_t)g >> 2) + 1, kSampleStream, w2);
+        auto word = [&](int k) { const int j = sh + k; return j < 4 ? pick4(w, j) : pick4(w2, j - 4); };
+        v.x = fmaf(v.x, s_a, gumbel_of(word(0)));
+        v.y = fmaf(v.y, s_a, gumbel_of(word(1)));
+        v.z = fmaf(v.z, s_a, gumbel_of(word(2)));
+        v.w = fmaf(v.w, s_a, gumbel_of(word(3)));
+        return v;
+    };
     auto allowed = [&](int c) { const int g = item_offset + c; return !arow || ((__ldg(arow + (g >> 5)) >> (g & 31)) & 1u); };
     // allow bits of the 4 scores of each segment of a trip, packed 4 per segment (all set when unrestricted)
     auto fetch_allow = [&](int base) {
@@ -428,9 +463,11 @@ __global__ void __launch_bounds__(kTopkWarps * 32) mask_topk_kernel(float* __res
     if constexpr (FILTER) cur_allow = fetch_allow(cs);
     {
         const bool h = lane < head && (!FILTER || allowed(c0 + lane));
-        top.offer(h ? row[c0 + lane] : -INFINITY, h ? item_offset + c0 + lane : -1);
+        float hv = h ? row[c0 + lane] : -INFINITY;
+        if constexpr (SAMPLE) if (sampled && h) hv = key1(hv, item_offset + c0 + lane);
+        top.offer(hv, h ? item_offset + c0 + lane : -1);
     }
-    bool probe = K <= 32 && c1v - cs >= kTopkSeg * 128;
+    bool probe = K <= 32 && c1v - cs >= kTopkSeg * 128 && !sampled;     // (the probe's bound holds for scores, not keys)
     for (int base = cs; base < c1v; base += kTopkSeg * 128) {
 #pragma unroll
         for (int q = 0; q < kTopkSeg; ++q) nxt[q] = fetch(base + kTopkSeg * 128 + q * 128);
@@ -467,11 +504,13 @@ __global__ void __launch_bounds__(kTopkWarps * 32) mask_topk_kernel(float* __res
             const int src = __ffs(__ballot_sync(0xffffffffu, rank == K - 1)) - 1;
             if (src >= 0) top.raise(__shfl_sync(0xffffffffu, m, src), __shfl_sync(0xffffffffu, mi, src) - 1);   // "- 1": that pair itself is admitted
         }
-        if (__any_sync(0xffffffffu, m >= top.thr_v)) {
+        if (__any_sync(0xffffffffu, bound(m) >= top.thr_v)) {
 #pragma unroll
             for (int q = 0; q < kTopkSeg; ++q) {
                 const int c = base + q * 128 + lane * 4;
-                unsigned bal = __ballot_sync(0xffffffffu, c < c1v && mq[q] >= top.thr_v);
+                const bool pass = c < c1v && bound(mq[q]) >= top.thr_v;
+                unsigned bal = __ballot_sync(0xffffffffu, pass);
+                if constexpr (SAMPLE) if (sampled && pass) cur[q] = key4(cur[q], item_offset + c);
                 while (bal) {
                     const int src = __ffs(bal) - 1;
                     bal &= bal - 1;
@@ -492,7 +531,9 @@ __global__ void __launch_bounds__(kTopkWarps * 32) mask_topk_kernel(float* __res
     {   // <= 3 tail columns
         const int c = c1v + lane;
         const bool t = c < c1 && (!FILTER || allowed(c));
-        top.offer(t ? row[c] : -INFINITY, t ? item_offset + c : -1);
+        float tv = t ? row[c] : -INFINITY;
+        if constexpr (SAMPLE) if (sampled && t) tv = key1(tv, item_offset + c);
+        top.offer(tv, t ? item_offset + c : -1);
     }
     float* ov = out_val + ((size_t)r * n_chunks + ch) * K;
     int32_t* oi = out_idx + ((size_t)r * n_chunks + ch) * K;
@@ -713,7 +754,8 @@ size_t hvae_mask_topk_chunks(int n_rows, int N) {
 
 static int mask_topk(float* S, int64_t lds, int n_rows, int N, int item_offset, const int64_t* indptr, const int32_t* indices,
                      const int32_t* rows, int exclude_seen, const uint32_t* allow, int64_t allow_stride, const int32_t* allow_of_row,
-                     int K, float* cand_val, int32_t* cand_idx, float* out_val, int32_t* out_idx, void* stream) {
+                     const float* row_inv_tau, const uint64_t* row_seed, int K, float* cand_val, int32_t* cand_idx, float* out_val,
+                     int32_t* out_idx, void* stream) {
     HVAE_REQUIRE(K >= 1 && K <= kMaxK, "mask_topk: K=%d outside [1,%d]", K, kMaxK);
     if (n_rows == 0) return 0;
     int nc, len;
@@ -723,13 +765,17 @@ static int mask_topk(float* S, int64_t lds, int n_rows, int N, int item_offset, 
     float* cv = nc == 1 ? out_val : cand_val;
     int32_t* ci = nc == 1 ? out_idx : cand_idx;
     const unsigned blocks = (unsigned)((units + kTopkWarps - 1) / kTopkWarps);
-    if (allow)
+    if (row_inv_tau)
+        launch_pdl(mask_topk_kernel<true, true>, blocks, kTopkWarps * 32, 0, (cudaStream_t)stream, S, lds, n_rows, N, item_offset, indptr,
+                   indices, rows, exclude_seen, K, nc, len, cv, ci, allow, allow_stride, allow_of_row, row_inv_tau, row_seed);
+    else if (allow)
         launch_pdl(mask_topk_kernel<true>, blocks, kTopkWarps * 32, 0, (cudaStream_t)stream, S, lds, n_rows, N, item_offset, indptr, indices,
-                   rows, exclude_seen, K, nc, len, cv, ci, allow, allow_stride, allow_of_row);
+                   rows, exclude_seen, K, nc, len, cv, ci, allow, allow_stride, allow_of_row, (const float*)nullptr, (const uint64_t*)nullptr);
     else
         launch_pdl(mask_topk_kernel<false>, blocks, kTopkWarps * 32, 0, (cudaStream_t)stream, S, lds, n_rows, N, item_offset, indptr, indices,
-                   rows, exclude_seen, K, nc, len, cv, ci, (const uint32_t*)nullptr, (int64_t)0, (const int32_t*)nullptr);
-    HVAE_LAUNCH_CHECK(allow ? "mask_topk_filtered" : "mask_topk");
+                   rows, exclude_seen, K, nc, len, cv, ci, (const uint32_t*)nullptr, (int64_t)0, (const int32_t*)nullptr, (const float*)nullptr,
+                   (const uint64_t*)nullptr);
+    HVAE_LAUNCH_CHECK(row_inv_tau ? "mask_topk_sampled" : allow ? "mask_topk_filtered" : "mask_topk");
     if (nc > 1) {
         launch_pdl(topk_merge_kernel, ceil_div(n_rows, kTopkWarps), kTopkWarps * 32, 0, (cudaStream_t)stream, (const float*)cv,
                    (const int32_t*)ci, n_rows, 1, nc * K, (int64_t)0, K, out_val, out_idx);
@@ -742,8 +788,8 @@ static int mask_topk(float* S, int64_t lds, int n_rows, int N, int item_offset, 
 int hvae_mask_topk(float* S, int64_t lds, int n_rows, int N, int item_offset, const int64_t* indptr, const int32_t* indices,
                    const int32_t* rows, int exclude_seen, int K, float* cand_val, int32_t* cand_idx, float* out_val, int32_t* out_idx,
                    void* stream) {
-    return mask_topk(S, lds, n_rows, N, item_offset, indptr, indices, rows, exclude_seen, nullptr, 0, nullptr, K, cand_val, cand_idx,
-                     out_val, out_idx, stream);
+    return mask_topk(S, lds, n_rows, N, item_offset, indptr, indices, rows, exclude_seen, nullptr, 0, nullptr, nullptr, nullptr, K,
+                     cand_val, cand_idx, out_val, out_idx, stream);
 }
 
 // The same restricted to per-row allow-sets (bitmaps over global item ids, see hvae_tc_score_topk_filtered); allow == NULL is
@@ -758,8 +804,25 @@ int hvae_mask_topk_filtered(float* S, int64_t lds, int n_rows, int N, int item_o
                      "mask_topk_filtered: allow_stride_words=%lld does not cover items up to %lld", (long long)allow_stride_words,
                      (long long)item_offset + N);
     }
-    return mask_topk(S, lds, n_rows, N, item_offset, indptr, indices, rows, exclude_seen, allow, allow_stride_words, allow_of_row, K,
-                     cand_val, cand_idx, out_val, out_idx, stream);
+    return mask_topk(S, lds, n_rows, N, item_offset, indptr, indices, rows, exclude_seen, allow, allow_stride_words, allow_of_row,
+                     nullptr, nullptr, K, cand_val, cand_idx, out_val, out_idx, stream);
+}
+
+// Gumbel-top-K sampling on top of hvae_mask_topk_filtered (see the header for the noise).  out_val holds the keys
+// s * row_inv_tau + g (s itself where row_inv_tau == 0); the caller takes the scores of the chosen ids from S.
+int hvae_mask_topk_sampled(float* S, int64_t lds, int n_rows, int N, int item_offset, const int64_t* indptr, const int32_t* indices,
+                           const int32_t* rows, int exclude_seen, const uint32_t* allow, int64_t allow_stride_words,
+                           const int32_t* allow_of_row, const float* row_inv_tau, const uint64_t* row_seed, int K, float* cand_val,
+                           int32_t* cand_idx, float* out_val, int32_t* out_idx, void* stream) {
+    HVAE_REQUIRE(row_inv_tau && row_seed, "mask_topk_sampled: row_inv_tau and row_seed are required");
+    if (allow) {
+        HVAE_REQUIRE(allow_of_row, "mask_topk_sampled: allow needs allow_of_row");
+        HVAE_REQUIRE(item_offset >= 0 && allow_stride_words >= ((int64_t)item_offset + N + 31) / 32,
+                     "mask_topk_sampled: allow_stride_words=%lld does not cover items up to %lld", (long long)allow_stride_words,
+                     (long long)item_offset + N);
+    }
+    return mask_topk(S, lds, n_rows, N, item_offset, indptr, indices, rows, exclude_seen, allow, allow_stride_words, allow_of_row,
+                     row_inv_tau, row_seed, K, cand_val, cand_idx, out_val, out_idx, stream);
 }
 
 int hvae_topk_merge(const float* cval, const int32_t* cidx, int n_rows, int GK, int K, float* out_val, int32_t* out_idx, void* stream) {

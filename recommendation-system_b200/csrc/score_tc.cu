@@ -48,6 +48,9 @@ struct StatsParams {
     const uint32_t* allow;        // [F, allow_stride] words
     int64_t allow_stride;
     const int32_t* allow_of_row;  // [B] bitmap row of each batch row, -1 = unrestricted
+    // TOPK with SAMPLE: Gumbel-top-K keys s / tau + g (common.cuh: gumbel_of) of rows with row_inv_tau != 0
+    const float* row_inv_tau;     // [B] 1 / tau, 0 = the row's plain scores
+    const uint64_t* row_seed;     // [B]
 };
 
 // One-pass mode (hvae_tc_score_onepass): softmax numerators are taken against a per-row shift c_b that does not depend on the
@@ -100,7 +103,11 @@ __device__ __forceinline__ void tile_allow_words(const uint32_t* arow, int g0, i
 // STG = operand ring depth; KREG > 0: top-K list of KREG >= K sorted keys per row in registers, KREG == 0: list in shared memory.
 // FILTER (TOPK only): a column is a candidate only if the row's allow bitmap has its bit; the words are ANDed into the
 // compare mask of each 32-column chunk, so a rejected column never reaches the insertion loop.
-template <int MODE, int STG, int KREG, bool FILTER = false>
+// SAMPLE (TOPK, with FILTER; P.allow may then be null): a row with row_inv_tau != 0 ranks the keys fmaf(s, inv_tau, g), g the
+// Gumbel noise of (row_seed, global item id).  The compare mask tests the bound fmaf(s, inv_tau, kGumbelMax) instead of s, so
+// Philox and the logarithms run only for the columns that pass it, once per group of 4 consecutive items.  The lists and the
+// written values hold keys.  A row with row_inv_tau == 0 runs the FILTER kernel's arithmetic on s itself.
+template <int MODE, int STG, int KREG, bool FILTER = false, bool SAMPLE = false>
 __global__ void __launch_bounds__(192, 1) score_stats_kernel(const __grid_constant__ CUtensorMap tmU,
                                                              const __grid_constant__ CUtensorMap tmE, StatsParams P) {
     constexpr int STAGES = STG;      // (shadows the file-level default)
@@ -204,8 +211,15 @@ __global__ void __launch_bounds__(192, 1) score_stats_kernel(const __grid_consta
         }
         const uint32_t* arow = nullptr;
         if constexpr (FILTER) {
-            const int f = row_ok ? P.allow_of_row[row] : -1;
+            const int f = row_ok && (!SAMPLE || P.allow) ? P.allow_of_row[row] : -1;
             if (f >= 0) arow = P.allow + (size_t)f * P.allow_stride;
+        }
+        // SAMPLE: candidate bound fmaf(v, s_a, s_b) (v itself for a deterministic row); the Philox words of item group nz_ctr
+        float s_a = 1.f, s_b = 0.f;
+        uint64_t seed = 0;
+        uint32_t nz[4] = {0u, 0u, 0u, 0u}, nz_ctr = 0xFFFFFFFFu;      // (gi >> 2 < 2^29: never a real group)
+        if constexpr (SAMPLE) {
+            if (row_ok && P.row_inv_tau[row] != 0.f) { s_a = P.row_inv_tau[row]; s_b = kGumbelMax; seed = P.row_seed[row]; }
         }
         for (int t = t0, ti = 0; t < t1; ++t, ++ti) {
             const int acc = ti & 1;
@@ -254,7 +268,10 @@ __global__ void __launch_bounds__(192, 1) score_stats_kernel(const __grid_consta
                     // code exists once, not 32 times (instruction-cache footprint), and v[j] is fetched by selects
                     unsigned mbits = 0;
 #pragma unroll
-                    for (int j = 0; j < 32; ++j) mbits |= (v[j] >= thr_v) ? (1u << j) : 0u;
+                    for (int j = 0; j < 32; ++j) {
+                        if constexpr (SAMPLE) mbits |= (fmaf(v[j], s_a, s_b) >= thr_v) ? (1u << j) : 0u;
+                        else mbits |= (v[j] >= thr_v) ? (1u << j) : 0u;
+                    }
                     const int left = n_valid - c * 32;
                     if (left < 32) mbits &= (1u << left) - 1u;
                     if constexpr (FILTER) {
@@ -271,6 +288,13 @@ __global__ void __launch_bounds__(192, 1) score_stats_kernel(const __grid_consta
 #pragma unroll
                         for (int t = 1; t < 32; ++t) x = (t == j) ? v[t] : x;
                         const int lc = c * 32 + j, gi = P.item_offset + col0 + lc;
+                        if constexpr (SAMPLE) {
+                            if (s_b != 0.f) {
+                                const uint32_t ctr = (uint32_t)gi >> 2;
+                                if (ctr != nz_ctr) { philox(seed, ctr, kSampleStream, nz); nz_ctr = ctr; }
+                                x = fmaf(x, s_a, gumbel_of(pick4(nz, gi & 3)));
+                            }
+                        }
                         uint64_t xk = 0;
                         if (KREG > 0) {
                             xk = topk_key(x, gi);
@@ -986,18 +1010,18 @@ static int pick_topk_splits(int m_tiles, int n_tiles) {
 constexpr size_t kStatsSmem = STAGES * STAGE_BYTES + 256 + 1024;                                        // LSE, register-list top-K
 constexpr size_t kStatsSmemList = STAGES_SMEM_LIST * STAGE_BYTES + 256 + BM * (MAXK_TC + 1) * 8 + 1024;   // shared-memory-list top-K
 
-// Sets the shared-memory limit of every top-K list bucket of one FILTER flavour (once per process).
-template <bool FILTER>
+// Sets the shared-memory limit of every top-K list bucket of one FILTER / SAMPLE flavour (once per process).
+template <bool FILTER, bool SAMPLE>
 static int topk_set_attrs() {
     static bool attr_set = false;
     if (!attr_set) {
-        HVAE_CUDA(cudaFuncSetAttribute(score_stats_kernel<MODE_TOPK, STAGES, 8, FILTER>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kStatsSmem));
-        HVAE_CUDA(cudaFuncSetAttribute(score_stats_kernel<MODE_TOPK, STAGES, 12, FILTER>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kStatsSmem));
-        HVAE_CUDA(cudaFuncSetAttribute(score_stats_kernel<MODE_TOPK, STAGES, 16, FILTER>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kStatsSmem));
-        HVAE_CUDA(cudaFuncSetAttribute(score_stats_kernel<MODE_TOPK, STAGES, 20, FILTER>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kStatsSmem));
-        HVAE_CUDA(cudaFuncSetAttribute(score_stats_kernel<MODE_TOPK, STAGES, 24, FILTER>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kStatsSmem));
-        HVAE_CUDA(cudaFuncSetAttribute(score_stats_kernel<MODE_TOPK, STAGES, 32, FILTER>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kStatsSmem));
-        HVAE_CUDA(cudaFuncSetAttribute(score_stats_kernel<MODE_TOPK, STAGES_SMEM_LIST, 0, FILTER>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+        HVAE_CUDA(cudaFuncSetAttribute(score_stats_kernel<MODE_TOPK, STAGES, 8, FILTER, SAMPLE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kStatsSmem));
+        HVAE_CUDA(cudaFuncSetAttribute(score_stats_kernel<MODE_TOPK, STAGES, 12, FILTER, SAMPLE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kStatsSmem));
+        HVAE_CUDA(cudaFuncSetAttribute(score_stats_kernel<MODE_TOPK, STAGES, 16, FILTER, SAMPLE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kStatsSmem));
+        HVAE_CUDA(cudaFuncSetAttribute(score_stats_kernel<MODE_TOPK, STAGES, 20, FILTER, SAMPLE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kStatsSmem));
+        HVAE_CUDA(cudaFuncSetAttribute(score_stats_kernel<MODE_TOPK, STAGES, 24, FILTER, SAMPLE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kStatsSmem));
+        HVAE_CUDA(cudaFuncSetAttribute(score_stats_kernel<MODE_TOPK, STAGES, 32, FILTER, SAMPLE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kStatsSmem));
+        HVAE_CUDA(cudaFuncSetAttribute(score_stats_kernel<MODE_TOPK, STAGES_SMEM_LIST, 0, FILTER, SAMPLE>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                        (int)kStatsSmemList));
         attr_set = true;
     }
@@ -1007,19 +1031,19 @@ static int topk_set_attrs() {
 // the list capacity is a compile-time size (register arrays): the smallest bucket that holds K.  A list longer than K costs twice: the
 // admission threshold is its LAST entry (more insertions) and every insertion walks the whole list -- hence buckets at the evaluation
 // protocol's own K values (5, 10, 20: src/ml/evaluate.py k_values)
-template <bool FILTER>
+template <bool FILTER, bool SAMPLE = false>
 static int launch_topk(int K, dim3 grid, cudaStream_t st, const CUtensorMap& tmU, const CUtensorMap& tmE, const StatsParams& P) {
-    if (int rc = topk_set_attrs<FILTER>()) return rc;
+    if (int rc = topk_set_attrs<FILTER, SAMPLE>()) return rc;
     static const int force_kreg = getenv("HVAE_TOPK_KREG") ? atoi(getenv("HVAE_TOPK_KREG")) : 0;        // A/B runs: a larger bucket than needed
     if (force_kreg >= K && force_kreg <= MAXK_REG) K = force_kreg;       // (P.K, the number of results written, stays)
-    if (K <= 8) launch_pdl(score_stats_kernel<MODE_TOPK, STAGES, 8, FILTER>, grid, 192, kStatsSmem, st, tmU, tmE, P);
-    else if (K <= 12) launch_pdl(score_stats_kernel<MODE_TOPK, STAGES, 12, FILTER>, grid, 192, kStatsSmem, st, tmU, tmE, P);
-    else if (K <= 16) launch_pdl(score_stats_kernel<MODE_TOPK, STAGES, 16, FILTER>, grid, 192, kStatsSmem, st, tmU, tmE, P);
-    else if (K <= 20) launch_pdl(score_stats_kernel<MODE_TOPK, STAGES, 20, FILTER>, grid, 192, kStatsSmem, st, tmU, tmE, P);
-    else if (K <= 24) launch_pdl(score_stats_kernel<MODE_TOPK, STAGES, 24, FILTER>, grid, 192, kStatsSmem, st, tmU, tmE, P);
-    else if (K <= MAXK_REG) launch_pdl(score_stats_kernel<MODE_TOPK, STAGES, 32, FILTER>, grid, 192, kStatsSmem, st, tmU, tmE, P);
-    else launch_pdl(score_stats_kernel<MODE_TOPK, STAGES_SMEM_LIST, 0, FILTER>, grid, 192, kStatsSmemList, st, tmU, tmE, P);
-    HVAE_LAUNCH_CHECK(FILTER ? "tc_score_topk_filtered" : "tc_score_topk");
+    if (K <= 8) launch_pdl(score_stats_kernel<MODE_TOPK, STAGES, 8, FILTER, SAMPLE>, grid, 192, kStatsSmem, st, tmU, tmE, P);
+    else if (K <= 12) launch_pdl(score_stats_kernel<MODE_TOPK, STAGES, 12, FILTER, SAMPLE>, grid, 192, kStatsSmem, st, tmU, tmE, P);
+    else if (K <= 16) launch_pdl(score_stats_kernel<MODE_TOPK, STAGES, 16, FILTER, SAMPLE>, grid, 192, kStatsSmem, st, tmU, tmE, P);
+    else if (K <= 20) launch_pdl(score_stats_kernel<MODE_TOPK, STAGES, 20, FILTER, SAMPLE>, grid, 192, kStatsSmem, st, tmU, tmE, P);
+    else if (K <= 24) launch_pdl(score_stats_kernel<MODE_TOPK, STAGES, 24, FILTER, SAMPLE>, grid, 192, kStatsSmem, st, tmU, tmE, P);
+    else if (K <= MAXK_REG) launch_pdl(score_stats_kernel<MODE_TOPK, STAGES, 32, FILTER, SAMPLE>, grid, 192, kStatsSmem, st, tmU, tmE, P);
+    else launch_pdl(score_stats_kernel<MODE_TOPK, STAGES_SMEM_LIST, 0, FILTER, SAMPLE>, grid, 192, kStatsSmemList, st, tmU, tmE, P);
+    HVAE_LAUNCH_CHECK(SAMPLE ? "tc_score_topk_sampled" : FILTER ? "tc_score_topk_filtered" : "tc_score_topk");
     return 0;
 }
 
@@ -1157,7 +1181,8 @@ int hvae_tc_score_lse_grad(const void* U, int ldu, int B, const void* E, int lde
 
 static int score_topk(const void* U, int ldu, int B, const void* E, int lde, int N, int d, int item_offset, const int64_t* indptr,
                       const int32_t* indices, const int32_t* rows, const uint32_t* allow, int64_t allow_stride,
-                      const int32_t* allow_of_row, int K, float* cand_val, int32_t* cand_idx, void* stream) {
+                      const int32_t* allow_of_row, const float* row_inv_tau, const uint64_t* row_seed, int K, float* cand_val,
+                      int32_t* cand_idx, void* stream) {
     if (B == 0) return 0;
     HVAE_REQUIRE(K >= 1 && K <= MAXK_TC, "tc_score_topk: K=%d outside [1,%d]", K, MAXK_TC);
     CUtensorMap tmU, tmE;
@@ -1171,7 +1196,9 @@ static int score_topk(const void* U, int ldu, int B, const void* E, int lde, int
     P.cand_val = cand_val; P.cand_idx = cand_idx;
     P.indptr = indptr; P.indices = indices; P.rows = rows;
     P.allow = allow; P.allow_stride = allow_stride; P.allow_of_row = allow_of_row;
+    P.row_inv_tau = row_inv_tau; P.row_seed = row_seed;
     const dim3 grid(m_tiles, P.n_splits);
+    if (row_inv_tau) return launch_topk<true, true>(K, grid, (cudaStream_t)stream, tmU, tmE, P);
     if (allow) return launch_topk<true>(K, grid, (cudaStream_t)stream, tmU, tmE, P);
     return launch_topk<false>(K, grid, (cudaStream_t)stream, tmU, tmE, P);
 }
@@ -1180,7 +1207,8 @@ static int score_topk(const void* U, int ldu, int B, const void* E, int lde, int
 // the caller reduces them with hvae_topk_merge.  K <= 128 (K <= 32: register-resident lists; above: shared-memory lists).
 int hvae_tc_score_topk(const void* U, int ldu, int B, const void* E, int lde, int N, int d, int item_offset, const int64_t* indptr,
                        const int32_t* indices, const int32_t* rows, int K, float* cand_val, int32_t* cand_idx, void* stream) {
-    return score_topk(U, ldu, B, E, lde, N, d, item_offset, indptr, indices, rows, nullptr, 0, nullptr, K, cand_val, cand_idx, stream);
+    return score_topk(U, ldu, B, E, lde, N, d, item_offset, indptr, indices, rows, nullptr, 0, nullptr, nullptr, nullptr, K, cand_val,
+                      cand_idx, stream);
 }
 
 // The same restricted to per-row allow-sets: row b may only return items whose bit is set in allow[allow_of_row[b]] (bitmaps over
@@ -1196,8 +1224,25 @@ int hvae_tc_score_topk_filtered(const void* U, int ldu, int B, const void* E, in
                      "tc_score_topk_filtered: allow_stride_words=%lld does not cover items up to %lld", (long long)allow_stride_words,
                      (long long)item_offset + N);
     }
-    return score_topk(U, ldu, B, E, lde, N, d, item_offset, indptr, indices, rows, allow, allow_stride_words, allow_of_row, K,
-                      cand_val, cand_idx, stream);
+    return score_topk(U, ldu, B, E, lde, N, d, item_offset, indptr, indices, rows, allow, allow_stride_words, allow_of_row, nullptr,
+                      nullptr, K, cand_val, cand_idx, stream);
+}
+
+// Gumbel-top-K sampling on top of hvae_tc_score_topk_filtered (see the header for the noise).  cand_val holds the keys
+// s * row_inv_tau + g (s itself where row_inv_tau == 0); merge with hvae_topk_merge, then take the scores of the chosen ids.
+int hvae_tc_score_topk_sampled(const void* U, int ldu, int B, const void* E, int lde, int N, int d, int item_offset,
+                               const int64_t* indptr, const int32_t* indices, const int32_t* rows, const uint32_t* allow,
+                               int64_t allow_stride_words, const int32_t* allow_of_row, const float* row_inv_tau,
+                               const uint64_t* row_seed, int K, float* cand_val, int32_t* cand_idx, void* stream) {
+    HVAE_REQUIRE(row_inv_tau && row_seed, "tc_score_topk_sampled: row_inv_tau and row_seed are required");
+    if (allow) {
+        HVAE_REQUIRE(allow_of_row, "tc_score_topk_sampled: allow needs allow_of_row");
+        HVAE_REQUIRE(item_offset >= 0 && allow_stride_words >= ((int64_t)item_offset + N + 31) / 32,
+                     "tc_score_topk_sampled: allow_stride_words=%lld does not cover items up to %lld", (long long)allow_stride_words,
+                     (long long)item_offset + N);
+    }
+    return score_topk(U, ldu, B, E, lde, N, d, item_offset, indptr, indices, rows, allow, allow_stride_words, allow_of_row,
+                      row_inv_tau, row_seed, K, cand_val, cand_idx, stream);
 }
 
 // 1 or 2 numerator sums per (split, row): the pair kernel's two CTAs each report the tiles they owned

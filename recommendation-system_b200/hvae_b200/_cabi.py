@@ -53,7 +53,7 @@ STATE_OFF = {name: getattr(StepState, name).offset // 4 for name, _ in StepState
 
 # Kernels of ours launched per C-ABI call (library-internal CUB passes are not counted); default 1.
 KERNELS_PER_CALL = {"hvae_ln_act_bwd": 2, "hvae_colsum": 2, "hvae_batch_transpose": 4, "hvae_grad_norm_clip": 2,
-                    "hvae_metrics_reduce": 2, "hvae_mask_topk": 2, "hvae_mask_topk_filtered": 2, "hvae_w1_plan": 2, "hvae_w1_grad": 2, "hvae_w1_max_work": 0, "hvae_w1_max_partial_rows": 0,
+                    "hvae_metrics_reduce": 2, "hvae_mask_topk": 2, "hvae_mask_topk_filtered": 2, "hvae_mask_topk_sampled": 2, "hvae_w1_plan": 2, "hvae_w1_grad": 2, "hvae_w1_max_work": 0, "hvae_w1_max_partial_rows": 0,
                     "hvae_tc_n_splits": 0, "hvae_tc_grad_splits": 0, "hvae_gemm_tf32_supported": 0, "hvae_tc_score_lse": 2, "hvae_tc_score_lse_grad": 2, "hvae_tc_onepass_subparts": 0, "hvae_h2d_csr_batch": 0, "hvae_d2h_floats": 0, "hvae_mask_topk_chunks": 0, "hvae_tc_topk_splits": 0, "hvae_last_error": 0, "hvae_abi_version": 0, "hvae_tc_duo_max_clusters": 0,
                     "hvae_ln_bwd_workspace_floats": 0, "hvae_batch_temp_bytes": 0}
 

@@ -22,6 +22,7 @@ from . import data as _data
 from ._cabi import p
 from .engine import Batch, DeviceCSR
 from .model import HybridVAE, create_hybrid_vae
+from .serve import check_seed, check_temperature
 
 logger = logging.getLogger(__name__)
 _build_input_matrix = _data.build_input_matrix
@@ -135,15 +136,21 @@ class RecommendationEvaluator:
         return indptr, (key % N).to(torch.int32)
 
     # -- batched primitives ----------------------------------------------------------------------------------------
-    def topk_users(self, user_indices, top_k: int, exclude_seen: bool = True, *, item_filter=None, exclude=None):
+    def topk_users(self, user_indices, top_k: int, exclude_seen: bool = True, *, item_filter=None, exclude=None,
+                   temperature=None, seed=None):
         """(values [n,K] f32, indices [n,K] int32) device tensors for the given users.
 
         item_filter: the name of a filter registered with add_item_filter, or one name (or None) per user: that user only gets
         items of the filter.  exclude: one array of item indices per user, left out on top of the seen items.  A user with
-        fewer than K admissible items gets (-inf, -1) in the remaining slots."""
+        fewer than K admissible items gets (-inf, -1) in the remaining slots.
+        temperature, seed: a scalar or one value per user (None = that user's plain top-K).  A user with a temperature tau
+        gets K items drawn without replacement from softmax(scores / tau) over the admissible items (Gumbel-top-K, noise of
+        (seed, item): the same arguments give the same draw in any batch and for any K, whose first k items are the k-item
+        draw), in drawn order, with their scores.  tau lies in [1e-3, 1e3], seeds in [0, 2^64); a tau needs a seed."""
         users = torch.as_tensor(np.asarray(user_indices, dtype=np.int32), device=self.device)
-        if item_filter is not None or exclude is not None:
-            return self._topk_filtered(users, top_k, exclude_seen, item_filter, exclude)
+        sample = self._sample_params(temperature, seed, users.shape[0])
+        if item_filter is not None or exclude is not None or sample is not None:
+            return self._topk_filtered(users, top_k, exclude_seen, item_filter, exclude, sample)
         eng = self.model.engine
         from . import tc
         if eng.precision != "fp32" and exclude_seen and top_k <= tc.MAX_K_REG and users.shape[0] >= 2 * self.batch_users:
@@ -168,7 +175,29 @@ class RecommendationEvaluator:
             return (torch.empty(0, top_k, device=self.device), torch.empty(0, top_k, dtype=torch.int32, device=self.device))
         return torch.cat(vals), torch.cat(idxs)
 
-    def _topk_filtered(self, users, top_k, exclude_seen, item_filter, exclude):
+    @staticmethod
+    def _per_user(x, n, what):
+        xs = [x] * n if x is None or np.ndim(x) == 0 else list(x)
+        if len(xs) != n:
+            raise ValueError(f"{what}: {len(xs)} entries for {n} users")
+        return xs
+
+    def _sample_params(self, temperature, seed, n):
+        """-> (inv_tau float32 [n], seed int64 [n]) host arrays (inv_tau 0 = plain top-K), or None when no user samples."""
+        if temperature is None:
+            return None
+        taus, seeds = self._per_user(temperature, n, "temperature"), self._per_user(seed, n, "seed")
+        inv_tau, seed64 = np.zeros(n, dtype=np.float32), np.zeros(n, dtype=np.uint64)
+        for r, (t, sd) in enumerate(zip(taus, seeds)):
+            if t is None:
+                continue
+            if sd is None:
+                raise ValueError("a temperature needs a seed")
+            inv_tau[r] = np.float32(1.0 / check_temperature(t))
+            seed64[r] = check_seed(sd)
+        return (inv_tau, seed64.view(np.int64)) if inv_tau.any() else None
+
+    def _topk_filtered(self, users, top_k, exclude_seen, item_filter, exclude, sample=None):
         n = users.shape[0]
         with self._filters_lock:
             table, filter_row = self._filters
@@ -182,6 +211,8 @@ class RecommendationEvaluator:
                 if e.size and (e.min() < 0 or e.max() >= self.n_items):
                     raise ValueError(f"exclude: item indices must lie in [0, {self.n_items})")
         aor_d = None if aor is None else torch.as_tensor(aor, device=self.device)
+        if sample is not None:
+            sample = tuple(torch.as_tensor(a, device=self.device) for a in sample)
         eng = self.model.engine
         vals, idxs = [], []
         with torch.no_grad():
@@ -189,7 +220,8 @@ class RecommendationEvaluator:
                 rows = users[s:s + self.batch_users].contiguous()
                 mask = None if exclude is None else self._mask_csr(rows, exclude[s:s + rows.shape[0]], exclude_seen)
                 allow = None if aor_d is None else (table, aor_d[s:s + rows.shape[0]].contiguous())
-                v, i = eng.topk(Batch(self._csr, rows, rows.shape[0], 1), top_k, exclude_seen, mask=mask, allow=allow)
+                smp = None if sample is None else tuple(a[s:s + rows.shape[0]].contiguous() for a in sample)
+                v, i = eng.topk(Batch(self._csr, rows, rows.shape[0], 1), top_k, exclude_seen, mask=mask, allow=allow, sample=smp)
                 vals.append(v)
                 idxs.append(i)
         if not vals:

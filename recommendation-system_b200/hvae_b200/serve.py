@@ -10,6 +10,9 @@ The FastAPI plumbing itself (routes, pydantic models, CORS) is out of scope: a h
 """
 from __future__ import annotations
 
+import math
+import numbers
+import random
 import threading
 import time
 from concurrent.futures import Future
@@ -18,10 +21,33 @@ from typing import Callable, Iterable, Sequence
 import numpy as np
 
 MAX_TOP_K = 100          # the API's own limit (src/api/server.py: RecommendationRequest.top_k <= 100)
+# Sampling temperatures: below 1e-3 the draw is the plain top-K wherever scores differ by more than 0.017, above 1e3 it is
+# close to uniform over the admissible items for any trained model; either end is better asked for without a temperature.
+MIN_TEMPERATURE, MAX_TEMPERATURE = 1e-3, 1e3
 
 
 class UnknownUser(KeyError):
     """The user id is not in the training data (the reference answers HTTP 404, server.py:134-138)."""
+
+
+def check_temperature(t) -> float:
+    """A sampling temperature as float; ValueError unless it is a finite real number in [MIN_TEMPERATURE, MAX_TEMPERATURE]."""
+    if isinstance(t, bool) or not isinstance(t, numbers.Real):
+        raise ValueError(f"temperature must be a number, got {t!r}")
+    t = float(t)
+    if not (math.isfinite(t) and MIN_TEMPERATURE <= t <= MAX_TEMPERATURE):
+        raise ValueError(f"temperature must lie in [{MIN_TEMPERATURE:g}, {MAX_TEMPERATURE:g}], got {t!r}")
+    return t
+
+
+def check_seed(seed) -> int:
+    """A sampling seed as int; ValueError unless it is an integer in [0, 2^64)."""
+    if isinstance(seed, bool) or not isinstance(seed, numbers.Integral):
+        raise ValueError(f"seed must be an integer, got {seed!r}")
+    seed = int(seed)
+    if not 0 <= seed < 1 << 64:
+        raise ValueError(f"seed must lie in [0, 2^64), got {seed}")
+    return seed
 
 
 def _response(user_id, idx: np.ndarray, val: np.ndarray, top_k: int, idx_to_item: dict, total_items: int) -> dict:
@@ -33,11 +59,19 @@ def _response(user_id, idx: np.ndarray, val: np.ndarray, top_k: int, idx_to_item
     return {"user_id": user_id, "recommendations": recs, "total_items": total_items}
 
 
+def _request_parts(req: tuple) -> tuple:
+    """(user_id, top_k, exclude_seen, item_filter, exclude_items, temperature, seed) of a 3- to 7-element request."""
+    if not 3 <= len(req) <= 7:
+        raise ValueError(f"a request has 3 to 7 elements, got {len(req)}")
+    return tuple(req) + (None,) * (7 - len(req))
+
+
 class RecommendService:
     """topk_fn(user_indices, K, exclude_seen) -> (values [n, K], indices [n, K]) array-likes; the production binding is
     `RecommendationEvaluator.topk_users` (`from_evaluator`).  A launch whose requests use item filters or exclusions calls
     topk_fn(user_indices, K, exclude_seen, item_filter=[name or None per row], exclude=[item index array per row]);
-    add_filter_fn(name, item_indices) registers an allow-set with the backend (RecommendationEvaluator.add_item_filter)."""
+    add_filter_fn(name, item_indices) registers an allow-set with the backend (RecommendationEvaluator.add_item_filter).
+    A launch with sampled requests also passes temperature=[tau or None per row], seed=[seed or None per row]."""
 
     def __init__(self, topk_fn: Callable, user_to_idx: dict, idx_to_item: dict, n_items: int, max_batch: int = 4096,
                  add_filter_fn: Callable | None = None):
@@ -46,6 +80,8 @@ class RecommendService:
         self.add_filter_fn = add_filter_fn
         self.filters: set = set()
         self._item_to_idx: dict | None = None
+        self._seeds = random.Random()         # seeds of sampled requests that bring none (OS entropy)
+        self._seeds_lock = threading.Lock()
 
     @classmethod
     def from_evaluator(cls, evaluator, idx_to_item: dict, max_batch: int = 4096):
@@ -93,46 +129,66 @@ class RecommendService:
         except TypeError as e:          # not iterable, or an unhashable id
             raise ValueError(f"exclude_items: {e}") from None
 
-    def recommend(self, user_id, top_k: int = 10, exclude_seen: bool = True, *, item_filter=None, exclude_items=()) -> dict:
-        out = self.recommend_many([(user_id, top_k, exclude_seen, item_filter, exclude_items)])[0]
+    def _new_seed(self) -> int:
+        with self._seeds_lock:
+            return self._seeds.getrandbits(53)       # (exact as a JSON number: a client can send it back unchanged)
+
+    def recommend(self, user_id, top_k: int = 10, exclude_seen: bool = True, *, item_filter=None, exclude_items=(),
+                  temperature=None, seed=None) -> dict:
+        """temperature: None for the top_k best items, else a sampled answer: top_k items drawn without replacement from
+        softmax(scores / temperature) (temperature in [MIN_TEMPERATURE, MAX_TEMPERATURE]), in drawn order.  seed: an
+        integer in [0, 2^64) (None: the service picks one); the response carries "temperature" and "seed", and the same
+        user, seed, temperature, filter, exclusions and model give the same answer."""
+        out = self.recommend_many([(user_id, top_k, exclude_seen, item_filter, exclude_items, temperature, seed)])[0]
         if isinstance(out, Exception):
             raise out
         return out
 
     def recommend_many(self, requests: Sequence[tuple]) -> list:
-        """requests: (user_id, top_k, exclude_seen[, item_filter[, exclude_items]]) tuples.  One launch per exclude_seen group
-        (K = the group's largest top_k), whatever filters and exclusions its requests carry.  Exclusions are API item ids; ids
-        without an item index are ignored (they can never be recommended).  Returns, in request order, the response dict or
-        the exception that request would have raised."""
+        """requests: (user_id, top_k, exclude_seen[, item_filter[, exclude_items[, temperature[, seed]]]]) tuples.  One launch
+        per exclude_seen group (K = the group's largest top_k), whatever filters, exclusions and temperatures its requests
+        carry.  Exclusions are API item ids; ids without an item index are ignored (they can never be recommended).  A request
+        with a temperature is sampled (see recommend).  Returns, in request order, the response dict or the exception that
+        request would have raised."""
         out: list = [None] * len(requests)
         groups: dict[bool, list[int]] = {}
         extra: dict[int, tuple] = {}         # request -> (filter name or None, excluded item indices)
+        sampled: dict[int, tuple] = {}       # request -> (temperature, seed)
         for n, req in enumerate(requests):
-            user_id, top_k, exclude_seen = req[:3]
-            item_filter = req[3] if len(req) > 3 else None
             try:
+                user_id, top_k, exclude_seen, item_filter, exclude_items, temperature, seed = _request_parts(req)
                 self._check(user_id, top_k, item_filter)
-                excluded = self._excluded(req[4] if len(req) > 4 else None)
+                excluded = self._excluded(exclude_items)
+                seed = None if seed is None else check_seed(seed)
+                if temperature is not None:
+                    temperature = check_temperature(temperature)
+                    seed = self._new_seed() if seed is None else seed
             except (UnknownUser, ValueError) as e:
                 out[n] = e
                 continue
             if item_filter is not None or len(excluded):
                 extra[n] = (item_filter, excluded)
+            if temperature is not None:
+                sampled[n] = (temperature, seed)
             groups.setdefault(bool(exclude_seen), []).append(n)
         for exclude_seen, members in groups.items():
             for s in range(0, len(members), self.max_batch):
                 part = members[s:s + self.max_batch]
                 K = min(max(int(requests[n][1]) for n in part), self.n_items)
                 users = np.array([self.user_to_idx[requests[n][0]] for n in part], dtype=np.int32)
+                kw = {}
                 if any(n in extra for n in part):
                     none = (None, np.zeros(0, dtype=np.int64))
-                    val, idx = self.topk_fn(users, K, exclude_seen, item_filter=[extra.get(n, none)[0] for n in part],
-                                            exclude=[extra.get(n, none)[1] for n in part])
-                else:
-                    val, idx = self.topk_fn(users, K, exclude_seen)
+                    kw.update(item_filter=[extra.get(n, none)[0] for n in part], exclude=[extra.get(n, none)[1] for n in part])
+                if any(n in sampled for n in part):
+                    kw.update(temperature=[sampled[n][0] if n in sampled else None for n in part],
+                              seed=[sampled[n][1] if n in sampled else None for n in part])
+                val, idx = self.topk_fn(users, K, exclude_seen, **kw)
                 val, idx = np.asarray(val), np.asarray(idx)
                 for r, n in enumerate(part):
                     out[n] = _response(requests[n][0], idx[r], val[r], int(requests[n][1]), self.idx_to_item, self.n_items)
+                    if n in sampled:
+                        out[n]["temperature"], out[n]["seed"] = sampled[n]
         return out
 
 
@@ -149,15 +205,20 @@ class MicroBatcher:
         self._thread = threading.Thread(target=self._run, name="hvae-microbatcher", daemon=True)
         self._thread.start()
 
-    def submit(self, user_id, top_k: int = 10, exclude_seen: bool = True, *, item_filter=None, exclude_items=()) -> Future:
+    def submit(self, user_id, top_k: int = 10, exclude_seen: bool = True, *, item_filter=None, exclude_items=(), temperature=None,
+               seed=None) -> Future:
         fut: Future = Future()
         if exclude_items is not None and not isinstance(exclude_items, (str, bytes)):
             try:
                 exclude_items = tuple(exclude_items)      # a copy: the caller may reuse its list
             except TypeError:
                 pass                                      # reported for this request by recommend_many
-        req = (user_id, top_k, exclude_seen) if item_filter is None and exclude_items in (None, ()) else \
-            (user_id, top_k, exclude_seen, item_filter, exclude_items)
+        if temperature is not None or seed is not None:
+            req = (user_id, top_k, exclude_seen, item_filter, exclude_items, temperature, seed)
+        elif item_filter is None and exclude_items in (None, ()):
+            req = (user_id, top_k, exclude_seen)
+        else:
+            req = (user_id, top_k, exclude_seen, item_filter, exclude_items)
         with self._cv:
             if self._closed:
                 raise RuntimeError("MicroBatcher is closed")

@@ -74,20 +74,24 @@ def score_loss_bf16(eng, batch, u, want_grad):
     return lse, dot, xsum, O, xsum
 
 
-def topk_bf16(eng, batch, u, K, exclude_seen, item_lo, item_hi, out_val, out_idx, mask=None, allow=None) -> bool:
+def topk_bf16(eng, batch, u, K, exclude_seen, item_lo, item_hi, out_val, out_idx, mask=None, allow=None, sample=None) -> bool:
     """Fused score + seen-mask + top-K over items [item_lo, item_hi).  False if K is beyond the fused kernel."""
     if K > MAX_K_TC:
         return False
     return topk_bf16_from_ub(eng, batch, user_vectors_bf16(eng, u, batch.B), K, exclude_seen, item_lo, item_hi, out_val, out_idx,
-                             mask, allow)
+                             mask, allow, sample)
 
 
-def topk_bf16_from_ub(eng, batch, ub, K, exclude_seen, item_lo, item_hi, out_val, out_idx, mask=None, allow=None) -> bool:
+def topk_bf16_from_ub(eng, batch, ub, K, exclude_seen, item_lo, item_hi, out_val, out_idx, mask=None, allow=None,
+                      sample=None) -> bool:
     """The same with the bf16 user vectors [B, r8(d)] already at hand (item-sharded evaluation all-gathers them).
 
     mask = (indptr int64 [B+1], indices int32): items to leave out, one sorted row per BATCH row; it replaces the batch's
     seen rows (exclude_seen is then not looked at).  allow = (bitmaps int32 [F, words], allow_of_row int32 [B]): row b only
-    returns items whose bit is set in bitmaps[allow_of_row[b]] (-1: unrestricted); slots it cannot fill hold (-inf, -1)."""
+    returns items whose bit is set in bitmaps[allow_of_row[b]] (-1: unrestricted); slots it cannot fill hold (-inf, -1).
+    sample = (inv_tau float32 [B], seed int64 [B]): row b with inv_tau[b] != 0 gets a K-item Gumbel-top-K draw from
+    softmax(scores / tau) (include/hvae_b200.h, hvae_tc_score_topk_sampled), in drawn order; out_val holds the drawn items'
+    scores.  Rows with inv_tau[b] == 0 get the deterministic top-K."""
     if K > MAX_K_TC:
         return False
     lay, ws, lib, st = eng.lay, eng.ws, eng.lib, eng.stream
@@ -100,7 +104,14 @@ def topk_bf16_from_ub(eng, batch, ub, K, exclude_seen, item_lo, item_hi, out_val
     ci = ws.get("tc_cand_i", (B, ns * K), torch.int32)
     csr = batch.csr
     with eng.span("score_topk"):
-        if mask is None and allow is None:
+        if sample is not None:
+            indptr, indices, rows = (mask[0], mask[1], None) if mask is not None else \
+                ((csr.indptr if exclude_seen else None), csr.indices, batch.rows)
+            bm, aor = allow if allow is not None else (None, None)
+            lib.tc_score_topk_sampled(p(ub), ld8, B, Eb.data_ptr() + 2 * item_lo * ld8, ld8, n_it, d, item_lo, p(indptr), p(indices),
+                                      p(rows), p(bm), 0 if bm is None else bm.stride(0), p(aor), p(sample[0]), p(sample[1]), K,
+                                      p(cv), p(ci), st)
+        elif mask is None and allow is None:
             lib.tc_score_topk(p(ub), ld8, B, Eb.data_ptr() + 2 * item_lo * ld8, ld8, n_it, d, item_lo,
                               p(csr.indptr) if exclude_seen else None, p(csr.indices), p(batch.rows), K, p(cv), p(ci), st)
         else:
@@ -112,4 +123,9 @@ def topk_bf16_from_ub(eng, batch, ub, K, exclude_seen, item_lo, item_hi, out_val
             lib.tc_score_topk_filtered(p(ub), ld8, B, Eb.data_ptr() + 2 * item_lo * ld8, ld8, n_it, d, item_lo, p(indptr), p(indices),
                                        p(rows), p(bm), 0 if bm is None else bm.stride(0), p(aor), K, p(cv), p(ci), st)
     lib.topk_merge(p(cv), p(ci), B, ns * K, K, p(out_val), p(out_idx), st)
+    if sample is not None:      # sampled rows hold keys: the drawn items' scores, from the same bf16 operands (id -1: -inf)
+        rank = ws.get("tc_sample_rank", (B,), torch.int32)
+        sc = ws.get("tc_sample_score", (B, K))
+        lib.candidate_rank(p(ub), ld8, p(Eb), ld8, d, 1, p(out_idx), K, B, p(sc), p(rank), st)
+        torch.where(sample[0][:, None] != 0, sc, out_val, out=out_val)
     return True
