@@ -191,6 +191,13 @@ int hvae_mask_topk_sampled(float* S, int64_t lds, int n_rows, int N, int item_of
                            int64_t allow_stride_words, const int32_t* allow_of_row, const float* row_inv_tau,
                            const uint64_t* row_seed, int K, float* cand_val, int32_t* cand_idx, float* out_val,
                            int32_t* out_idx, void* stream);
+/* The same, boosted (see hvae_tc_score_topk_boosted).  out_val holds keys: take the chosen ids' scores from S. */
+int hvae_mask_topk_boosted(float* S, int64_t lds, int n_rows, int N, int item_offset, const int64_t* indptr,
+                           const int32_t* indices, const int32_t* rows, int exclude_seen, const uint32_t* allow,
+                           int64_t allow_stride_words, const int32_t* allow_of_row, const float* row_inv_tau,
+                           const uint64_t* row_seed, const float* boost, int64_t boost_stride, const float* boost_bound,
+                           int64_t bound_stride, const int32_t* boost_of_row, const float* row_boost_weight, int K,
+                           float* cand_val, int32_t* cand_idx, float* out_val, int32_t* out_idx, void* stream);
 int hvae_topk_merge(const float* cval, const int32_t* cidx, int n_rows, int GK, int K, float* out_val, int32_t* out_idx,
                     void* stream);
 /* The same merge over the blocks of an all-gather, read in place: rank g's K candidates of row r are at
@@ -242,6 +249,24 @@ int hvae_tc_score_topk_sampled(const void* U, int ldu, int B, const void* E, int
                                const int64_t* indptr, const int32_t* indices, const int32_t* rows,
                                const uint32_t* allow, int64_t allow_stride_words, const int32_t* allow_of_row,
                                const float* row_inv_tau, const uint64_t* row_seed, int K, float* cand_val,
+                               int32_t* cand_idx, void* stream);
+/* The same, boosted: a boost is a finite fp32 vector beta_v over GLOBAL item ids, row v of boost [V, boost_stride]
+ * (boost_stride >= item_offset + N).  Row b with boost_of_row[b] = v >= 0 and w = row_boost_weight[b] != 0 ranks the keys
+ *     k_bi = fmaf(w, beta_v[i], s_bi)        (s the score the kernel computes)
+ * under the order (key desc, global id desc); sampled too (row_inv_tau[b] != 0), it ranks fmaf(k_bi, row_inv_tau[b], g_i)
+ * with the noise above, so its K best are a draw from softmax((s + w beta) / tau).  Seen, excluded and disallowed items are
+ * never returned.  A row with w == 0 or boost_of_row[b] == -1 gets exactly what hvae_tc_score_topk_sampled gives it (and
+ * hvae_tc_score_topk_filtered when row_inv_tau == NULL, which means no row is sampled; row_seed may then be NULL too).
+ * boost_bound [V, bound_stride] (bound_stride >= 2 * ceil((item_offset + N) / 32)) holds, for each aligned 32-item block j
+ * of global ids, (max, min) of beta_v over the block at [2j], [2j + 1]; the kernels prune with it and stay exact only if it
+ * is right.  cand_val holds KEYS (merge with hvae_topk_merge); the caller puts back the scores of the chosen items.
+ * boost == NULL is hvae_tc_score_topk_sampled.  Meant for |beta| <= 1e6 and |w| <= 1e3, so that keys stay finite. */
+int hvae_tc_score_topk_boosted(const void* U, int ldu, int B, const void* E, int lde, int N, int d, int item_offset,
+                               const int64_t* indptr, const int32_t* indices, const int32_t* rows,
+                               const uint32_t* allow, int64_t allow_stride_words, const int32_t* allow_of_row,
+                               const float* row_inv_tau, const uint64_t* row_seed, const float* boost,
+                               int64_t boost_stride, const float* boost_bound, int64_t bound_stride,
+                               const int32_t* boost_of_row, const float* row_boost_weight, int K, float* cand_val,
                                int32_t* cand_idx, void* stream);
 
 /* Backward through the scores: O[b,:] = sum_i softmax(S_b)_i E_i with S recomputed on the tensor cores

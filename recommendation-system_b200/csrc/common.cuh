@@ -104,6 +104,42 @@ __device__ __forceinline__ uint32_t pick4(const uint32_t (&w)[4], int k) {
     return k == 0 ? w[0] : k == 1 ? w[1] : k == 2 ? w[2] : w[3];
 }
 
+// ---- Boosted top-K (include/hvae_b200.h, hvae_tc_score_topk_boosted): score thresholds for exact pruning ----
+// A boosted row ranks k = fmaf(w, beta_i, s) (and, sampled, fmaf(k, inv_tau, g)).  The kernels compare each score s with one
+// threshold per group of columns, the list threshold thr carried back through the key's roundings.  With round() the fp32
+// rounding to nearest, which is monotone, and pred(T) the float below T: round(x) >= T implies x > pred(T) (an x <= pred(T)
+// rounds to at most pred(T)).  The derivations start from key >= thr, so a key that ties the threshold (and may win on its id)
+// passes; the result of sample_threshold is a bound on k, fed to boost_threshold as T for a row that is both.
+// sample_threshold: key = round(k*a + g) >= thr, g <= kGumbelMax, a = inv_tau > 0
+//     => k*a > pred(thr) - kGumbelMax >= D = fsub_rd(pred(thr), kGumbelMax)  =>  k > D/a >= fdiv_rd(D, a).
+// boost_threshold: k = round(s + w*beta_i) >= T, w*beta_i <= bplus (bplus rounded up from w * the block max, or w * the
+// block min when w < 0)  =>  s + bplus > pred(T)  =>  s > pred(T) - bplus >= fsub_rd(pred(T), bplus).
+// thr = -inf gives -inf in both (every column passes).  A column below the result can never enter the list; the list itself
+// is then updated with the exactly computed key, so the result only decides how much arithmetic runs.
+__device__ __forceinline__ float sample_threshold(float thr, float inv_tau) {
+    return __fdiv_rd(__fsub_rd(nextafterf(thr, -INFINITY), kGumbelMax), inv_tau);
+}
+__device__ __forceinline__ float boost_threshold(float T, float bplus) { return __fsub_rd(nextafterf(T, -INFINITY), bplus); }
+// bplus of the columns in blocks with extremes e0, e1 (block maxima when w >= 0, minima when w < 0; e0 == e1 for one block)
+__device__ __forceinline__ float boost_bplus(float w, float e0, float e1) {
+    return __fmul_ru(w, w >= 0.f ? fmaxf(e0, e1) : fminf(e0, e1));
+}
+// The boost arguments of hvae_tc_score_topk_boosted / hvae_mask_topk_boosted.
+struct BoostArgs {
+    const float* boost; int64_t boost_stride;
+    const float* bound; int64_t bound_stride;
+    const int32_t* boost_of_row; const float* row_weight;
+};
+// 0, or hvae_fail's status when the tables do not cover the global ids item_offset .. item_offset + N - 1
+inline int check_boost_args(const char* what, const BoostArgs& b, int item_offset, int N) {
+    const int64_t end = (int64_t)item_offset + N;
+    HVAE_REQUIRE(b.bound && b.boost_of_row && b.row_weight, "%s: boost needs boost_bound, boost_of_row and row_boost_weight", what);
+    HVAE_REQUIRE(item_offset >= 0 && b.boost_stride >= end && b.bound_stride >= 2 * ((end + 31) / 32),
+                 "%s: boost_stride=%lld / bound_stride=%lld do not cover items up to %lld", what, (long long)b.boost_stride,
+                 (long long)b.bound_stride, (long long)end);
+    return 0;
+}
+
 __host__ __device__ __forceinline__ int ceil_div(int a, int b) { return (a + b - 1) / b; }
 __host__ __device__ __forceinline__ int round_up(int a, int b) { return (a + b - 1) / b * b; }
 

@@ -374,7 +374,13 @@ constexpr int kTopkSeg = 8;          // 512-byte row segments per trip of the sc
 // segment tests take the bound fmaf(max, inv_tau, kGumbelMax) instead of the maximum, and only a lane whose segment passes
 // runs Philox (its 4 scores are one counter when the global id of the segment is a multiple of 4, else two) and the logs.
 // The probe is skipped for such rows.  A row with row_inv_tau[r] == 0 runs the FILTER kernel's arithmetic.
-template <bool FILTER, bool SAMPLE = false>
+// BOOST (with FILTER and SAMPLE; allow and row_inv_tau may then be null): a row with a boost and w != 0 ranks
+// fmaf(w, beta[g], s) (then the Gumbel key of that if sampled).  Each lane fetches, with the next trip's scores, the bound
+// table entries of the one or two 32-item blocks each of its segments touches, and tests the segment's maximum against a
+// score threshold derived from the list's and the segment's bound on w*beta (common.cuh: sample_threshold,
+// boost_threshold); beta is read only for segments that pass.  The probe is skipped for boosted rows.  A row without a
+// boost gets what the SAMPLE kernel gives it: the thresholds only prune, the list takes the same exact keys.
+template <bool FILTER, bool SAMPLE = false, bool BOOST = false>
 __global__ void __launch_bounds__(kTopkWarps * 32) mask_topk_kernel(float* __restrict__ S, int64_t lds, int n_rows, int N,
                                                                     int item_offset, const int64_t* __restrict__ indptr,
                                                                     const int32_t* __restrict__ indices,
@@ -383,7 +389,7 @@ __global__ void __launch_bounds__(kTopkWarps * 32) mask_topk_kernel(float* __res
                                                                     int32_t* __restrict__ out_idx, const uint32_t* __restrict__ allow,
                                                                     int64_t allow_stride, const int32_t* __restrict__ allow_of_row,
                                                                     const float* __restrict__ row_inv_tau,
-                                                                    const uint64_t* __restrict__ row_seed) {
+                                                                    const uint64_t* __restrict__ row_seed, BoostArgs bst) {
     pdl_prologue();
     __shared__ float sv_all[kTopkWarps][kMaxK];
     __shared__ int si_all[kTopkWarps][kMaxK];
@@ -418,9 +424,40 @@ __global__ void __launch_bounds__(kTopkWarps * 32) mask_topk_kernel(float* __res
     float s_a = 1.f, s_b = 0.f;     // SAMPLE: candidate bound fmaf(v, s_a, s_b)
     uint64_t seed = 0;
     if constexpr (SAMPLE) {
-        if (row_inv_tau[r] != 0.f) { s_a = row_inv_tau[r]; s_b = kGumbelMax; seed = row_seed[r]; }
+        if ((!BOOST || row_inv_tau) && row_inv_tau[r] != 0.f) { s_a = row_inv_tau[r]; s_b = kGumbelMax; seed = row_seed[r]; }
     }
     const bool sampled = SAMPLE && s_b != 0.f;
+    // BOOST: the row's beta (null: no boost), weight, and bound table at its block maxima (w >= 0) or minima (w < 0)
+    const float* brow = nullptr;
+    const float* bext = nullptr;
+    float bw = 0.f;
+    if constexpr (BOOST) {
+        const int bv = bst.boost_of_row[r];
+        if (bv >= 0 && bst.row_weight[r] != 0.f) {
+            bw = bst.row_weight[r];
+            brow = bst.boost + (size_t)bv * bst.boost_stride;
+            bext = bst.bound + (size_t)bv * bst.bound_stride + (bw >= 0.f ? 0 : 1);
+        }
+    }
+    const bool boosted = BOOST && brow;
+    auto boost1 = [&](float x, int g) { return boosted ? fmaf(bw, __ldg(brow + g), x) : x; };
+    auto boost4 = [&](float4 v, int g) {     // the 4 items g..g+3
+        v.x = fmaf(bw, __ldg(brow + g), v.x);
+        v.y = fmaf(bw, __ldg(brow + g + 1), v.y);
+        v.z = fmaf(bw, __ldg(brow + g + 2), v.z);
+        v.w = fmaf(bw, __ldg(brow + g + 3), v.w);
+        return v;
+    };
+    // bound table entries of the first and the last block each segment of a trip touches (read at the next trip)
+    auto fetch_bound = [&](int base, float (&e0)[kTopkSeg], float (&e1)[kTopkSeg]) {
+#pragma unroll
+        for (int q = 0; q < kTopkSeg; ++q) {
+            const int c = base + q * 128 + lane * 4, g = item_offset + c;
+            const bool in = boosted && base < c1v && c < c1v;
+            e0[q] = in ? __ldg(bext + 2 * (size_t)(g >> 5)) : 0.f;
+            e1[q] = in && (g & 31) > 28 ? __ldg(bext + 2 * (size_t)((g + 3) >> 5)) : e0[q];
+        }
+    };
     auto bound = [&](float x) { if constexpr (SAMPLE) return fmaf(x, s_a, s_b); else return x; };
     auto key1 = [&](float x, int g) {
         uint32_t w[4];
@@ -464,13 +501,17 @@ __global__ void __launch_bounds__(kTopkWarps * 32) mask_topk_kernel(float* __res
     {
         const bool h = lane < head && (!FILTER || allowed(c0 + lane));
         float hv = h ? row[c0 + lane] : -INFINITY;
+        if constexpr (BOOST) if (h) hv = boost1(hv, item_offset + c0 + lane);
         if constexpr (SAMPLE) if (sampled && h) hv = key1(hv, item_offset + c0 + lane);
         top.offer(hv, h ? item_offset + c0 + lane : -1);
     }
-    bool probe = K <= 32 && c1v - cs >= kTopkSeg * 128 && !sampled;     // (the probe's bound holds for scores, not keys)
+    float cur_e0[kTopkSeg], cur_e1[kTopkSeg], nxt_e0[kTopkSeg], nxt_e1[kTopkSeg];
+    if constexpr (BOOST) fetch_bound(cs, cur_e0, cur_e1);
+    bool probe = K <= 32 && c1v - cs >= kTopkSeg * 128 && !sampled && !boosted;     // (the probe's bound holds for scores, not keys)
     for (int base = cs; base < c1v; base += kTopkSeg * 128) {
 #pragma unroll
         for (int q = 0; q < kTopkSeg; ++q) nxt[q] = fetch(base + kTopkSeg * 128 + q * 128);
+        if constexpr (BOOST) fetch_bound(base + kTopkSeg * 128, nxt_e0, nxt_e1);
         if constexpr (FILTER) {
             nxt_allow = fetch_allow(base + kTopkSeg * 128);
 #pragma unroll
@@ -504,12 +545,22 @@ __global__ void __launch_bounds__(kTopkWarps * 32) mask_topk_kernel(float* __res
             const int src = __ffs(__ballot_sync(0xffffffffu, rank == K - 1)) - 1;
             if (src >= 0) top.raise(__shfl_sync(0xffffffffu, m, src), __shfl_sync(0xffffffffu, mi, src) - 1);   // "- 1": that pair itself is admitted
         }
-        if (__any_sync(0xffffffffu, bound(m) >= top.thr_v)) {
+        unsigned seg_pass = 0;      // BOOST: the segments that pass their score threshold
+        if constexpr (BOOST) {
+            const float T = sampled ? sample_threshold(top.thr_v, s_a) : top.thr_v;
+#pragma unroll
+            for (int q = 0; q < kTopkSeg; ++q) {
+                const float thr_q = boosted ? boost_threshold(T, boost_bplus(bw, cur_e0[q], cur_e1[q])) : T;
+                seg_pass |= (base + q * 128 + lane * 4 < c1v && mq[q] >= thr_q) ? 1u << q : 0u;
+            }
+        }
+        if (__any_sync(0xffffffffu, BOOST ? seg_pass != 0 : bound(m) >= top.thr_v)) {
 #pragma unroll
             for (int q = 0; q < kTopkSeg; ++q) {
                 const int c = base + q * 128 + lane * 4;
-                const bool pass = c < c1v && bound(mq[q]) >= top.thr_v;
+                const bool pass = BOOST ? ((seg_pass >> q) & 1u) != 0 : c < c1v && bound(mq[q]) >= top.thr_v;
                 unsigned bal = __ballot_sync(0xffffffffu, pass);
+                if constexpr (BOOST) if (boosted && pass) cur[q] = boost4(cur[q], item_offset + c);
                 if constexpr (SAMPLE) if (sampled && pass) cur[q] = key4(cur[q], item_offset + c);
                 while (bal) {
                     const int src = __ffs(bal) - 1;
@@ -527,11 +578,16 @@ __global__ void __launch_bounds__(kTopkWarps * 32) mask_topk_kernel(float* __res
 #pragma unroll
         for (int q = 0; q < kTopkSeg; ++q) cur[q] = nxt[q];
         if constexpr (FILTER) cur_allow = nxt_allow;
+        if constexpr (BOOST) {
+#pragma unroll
+            for (int q = 0; q < kTopkSeg; ++q) { cur_e0[q] = nxt_e0[q]; cur_e1[q] = nxt_e1[q]; }
+        }
     }
     {   // <= 3 tail columns
         const int c = c1v + lane;
         const bool t = c < c1 && (!FILTER || allowed(c));
         float tv = t ? row[c] : -INFINITY;
+        if constexpr (BOOST) if (t) tv = boost1(tv, item_offset + c);
         if constexpr (SAMPLE) if (sampled && t) tv = key1(tv, item_offset + c);
         top.offer(tv, t ? item_offset + c : -1);
     }
@@ -755,7 +811,7 @@ size_t hvae_mask_topk_chunks(int n_rows, int N) {
 static int mask_topk(float* S, int64_t lds, int n_rows, int N, int item_offset, const int64_t* indptr, const int32_t* indices,
                      const int32_t* rows, int exclude_seen, const uint32_t* allow, int64_t allow_stride, const int32_t* allow_of_row,
                      const float* row_inv_tau, const uint64_t* row_seed, int K, float* cand_val, int32_t* cand_idx, float* out_val,
-                     int32_t* out_idx, void* stream) {
+                     int32_t* out_idx, void* stream, const BoostArgs* bst = nullptr) {
     HVAE_REQUIRE(K >= 1 && K <= kMaxK, "mask_topk: K=%d outside [1,%d]", K, kMaxK);
     if (n_rows == 0) return 0;
     int nc, len;
@@ -765,17 +821,21 @@ static int mask_topk(float* S, int64_t lds, int n_rows, int N, int item_offset, 
     float* cv = nc == 1 ? out_val : cand_val;
     int32_t* ci = nc == 1 ? out_idx : cand_idx;
     const unsigned blocks = (unsigned)((units + kTopkWarps - 1) / kTopkWarps);
-    if (row_inv_tau)
+    if (bst)
+        launch_pdl(mask_topk_kernel<true, true, true>, blocks, kTopkWarps * 32, 0, (cudaStream_t)stream, S, lds, n_rows, N, item_offset,
+                   indptr, indices, rows, exclude_seen, K, nc, len, cv, ci, allow, allow_stride, allow_of_row, row_inv_tau, row_seed, *bst);
+    else if (row_inv_tau)
         launch_pdl(mask_topk_kernel<true, true>, blocks, kTopkWarps * 32, 0, (cudaStream_t)stream, S, lds, n_rows, N, item_offset, indptr,
-                   indices, rows, exclude_seen, K, nc, len, cv, ci, allow, allow_stride, allow_of_row, row_inv_tau, row_seed);
+                   indices, rows, exclude_seen, K, nc, len, cv, ci, allow, allow_stride, allow_of_row, row_inv_tau, row_seed, BoostArgs{});
     else if (allow)
         launch_pdl(mask_topk_kernel<true>, blocks, kTopkWarps * 32, 0, (cudaStream_t)stream, S, lds, n_rows, N, item_offset, indptr, indices,
-                   rows, exclude_seen, K, nc, len, cv, ci, allow, allow_stride, allow_of_row, (const float*)nullptr, (const uint64_t*)nullptr);
+                   rows, exclude_seen, K, nc, len, cv, ci, allow, allow_stride, allow_of_row, (const float*)nullptr, (const uint64_t*)nullptr,
+                   BoostArgs{});
     else
         launch_pdl(mask_topk_kernel<false>, blocks, kTopkWarps * 32, 0, (cudaStream_t)stream, S, lds, n_rows, N, item_offset, indptr, indices,
                    rows, exclude_seen, K, nc, len, cv, ci, (const uint32_t*)nullptr, (int64_t)0, (const int32_t*)nullptr, (const float*)nullptr,
-                   (const uint64_t*)nullptr);
-    HVAE_LAUNCH_CHECK(row_inv_tau ? "mask_topk_sampled" : allow ? "mask_topk_filtered" : "mask_topk");
+                   (const uint64_t*)nullptr, BoostArgs{});
+    HVAE_LAUNCH_CHECK(bst ? "mask_topk_boosted" : row_inv_tau ? "mask_topk_sampled" : allow ? "mask_topk_filtered" : "mask_topk");
     if (nc > 1) {
         launch_pdl(topk_merge_kernel, ceil_div(n_rows, kTopkWarps), kTopkWarps * 32, 0, (cudaStream_t)stream, (const float*)cv,
                    (const int32_t*)ci, n_rows, 1, nc * K, (int64_t)0, K, out_val, out_idx);
@@ -823,6 +883,30 @@ int hvae_mask_topk_sampled(float* S, int64_t lds, int n_rows, int N, int item_of
     }
     return mask_topk(S, lds, n_rows, N, item_offset, indptr, indices, rows, exclude_seen, allow, allow_stride_words, allow_of_row,
                      row_inv_tau, row_seed, K, cand_val, cand_idx, out_val, out_idx, stream);
+}
+
+// Boosted top-K on top of hvae_mask_topk_sampled (see hvae_tc_score_topk_boosted): out_val holds keys, the caller takes the
+// scores of the chosen ids from S.  row_inv_tau / row_seed may be NULL; boost == NULL is hvae_mask_topk_sampled, or
+// hvae_mask_topk_filtered without row_inv_tau.
+int hvae_mask_topk_boosted(float* S, int64_t lds, int n_rows, int N, int item_offset, const int64_t* indptr, const int32_t* indices,
+                           const int32_t* rows, int exclude_seen, const uint32_t* allow, int64_t allow_stride_words,
+                           const int32_t* allow_of_row, const float* row_inv_tau, const uint64_t* row_seed, const float* boost,
+                           int64_t boost_stride, const float* boost_bound, int64_t bound_stride, const int32_t* boost_of_row,
+                           const float* row_boost_weight, int K, float* cand_val, int32_t* cand_idx, float* out_val, int32_t* out_idx,
+                           void* stream) {
+    HVAE_REQUIRE(!row_inv_tau || row_seed, "mask_topk_boosted: row_inv_tau needs row_seed");
+    if (allow) {
+        HVAE_REQUIRE(allow_of_row, "mask_topk_boosted: allow needs allow_of_row");
+        HVAE_REQUIRE(item_offset >= 0 && allow_stride_words >= ((int64_t)item_offset + N + 31) / 32,
+                     "mask_topk_boosted: allow_stride_words=%lld does not cover items up to %lld", (long long)allow_stride_words,
+                     (long long)item_offset + N);
+    }
+    const BoostArgs bst{boost, boost_stride, boost_bound, bound_stride, boost_of_row, row_boost_weight};
+    if (boost) {
+        if (int rc = check_boost_args("mask_topk_boosted", bst, item_offset, N)) return rc;
+    }
+    return mask_topk(S, lds, n_rows, N, item_offset, indptr, indices, rows, exclude_seen, allow, allow_stride_words, allow_of_row,
+                     row_inv_tau, row_seed, K, cand_val, cand_idx, out_val, out_idx, stream, boost ? &bst : nullptr);
 }
 
 int hvae_topk_merge(const float* cval, const int32_t* cidx, int n_rows, int GK, int K, float* out_val, int32_t* out_idx, void* stream) {

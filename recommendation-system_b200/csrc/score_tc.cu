@@ -12,6 +12,7 @@
 // Roofline: tensor pipe (2*128*256*d flop per tile); HBM traffic is E once (L2 serves the re-reads across user tiles).
 #include <cfloat>
 #include <cstdlib>
+#include <type_traits>
 
 #include "common.cuh"
 #include "hvae_b200.h"
@@ -51,6 +52,16 @@ struct StatsParams {
     // TOPK with SAMPLE: Gumbel-top-K keys s / tau + g (common.cuh: gumbel_of) of rows with row_inv_tau != 0
     const float* row_inv_tau;     // [B] 1 / tau, 0 = the row's plain scores
     const uint64_t* row_seed;     // [B]
+};
+// TOPK with BOOST: rows with a boost rank fmaf(w, beta[i], s) (before the Gumbel noise of a sampled row).  A type of its own, so
+// that the other instantiations keep their parameter block (and their code) as it is.
+struct BoostStatsParams : StatsParams {
+    const float* boost;           // [V, boost_stride] beta over global item ids
+    int64_t boost_stride;
+    const float* boost_bound;     // [V, bound_stride]: (max, min) of beta over each aligned 32-item block of global ids
+    int64_t bound_stride;
+    const int32_t* boost_of_row;  // [B] boost of each batch row, -1 = none
+    const float* row_boost_weight;  // [B] w, 0 = no boost
 };
 
 // One-pass mode (hvae_tc_score_onepass): softmax numerators are taken against a per-row shift c_b that does not depend on the
@@ -100,6 +111,18 @@ __device__ __forceinline__ void tile_allow_words(const uint32_t* arow, int g0, i
     for (int e = 0; e < 8; ++e) aw[e] = __funnelshift_r(raw[e], raw[e + 1], sh);
 }
 
+// bplus (common.cuh: boost_bplus) of the eight 32-column chunks of the tile of items g0.. of a boosted row; bext = the row's
+// bound table shifted to its block maxima (w >= 0) or minima (w < 0), stride 2 per block.  Chunk c covers block (g0 >> 5) + c
+// and, when g0 is not a multiple of 32, the next one; blocks past the one holding item g_end - 1 are replaced by that one.
+__device__ __forceinline__ void tile_boost_bplus(const float* bext, float w, int g0, int g_end, float (&bp)[8]) {
+    const int w0 = g0 >> 5, wlast = (g_end - 1) >> 5;
+    float raw[9];
+#pragma unroll
+    for (int e = 0; e < 9; ++e) raw[e] = __ldg(bext + 2 * (size_t)min(w0 + e, wlast));
+#pragma unroll
+    for (int e = 0; e < 8; ++e) bp[e] = boost_bplus(w, raw[e], (g0 & 31) ? raw[e + 1] : raw[e]);
+}
+
 // STG = operand ring depth; KREG > 0: top-K list of KREG >= K sorted keys per row in registers, KREG == 0: list in shared memory.
 // FILTER (TOPK only): a column is a candidate only if the row's allow bitmap has its bit; the words are ANDed into the
 // compare mask of each 32-column chunk, so a rejected column never reaches the insertion loop.
@@ -107,9 +130,15 @@ __device__ __forceinline__ void tile_allow_words(const uint32_t* arow, int g0, i
 // Gumbel noise of (row_seed, global item id).  The compare mask tests the bound fmaf(s, inv_tau, kGumbelMax) instead of s, so
 // Philox and the logarithms run only for the columns that pass it, once per group of 4 consecutive items.  The lists and the
 // written values hold keys.  A row with row_inv_tau == 0 runs the FILTER kernel's arithmetic on s itself.
-template <int MODE, int STG, int KREG, bool FILTER = false, bool SAMPLE = false>
+// BOOST (TOPK, with FILTER and SAMPLE; P.allow and P.row_inv_tau may then be null): a row with a boost and w != 0 ranks
+// fmaf(w, beta[i], s) (then the Gumbel key of that if sampled).  Each 32-column chunk compares the raw scores with one score
+// threshold derived from the list's (common.cuh: sample_threshold, boost_threshold), using the chunk's bound on w*beta from
+// the block table (loaded per tile, during the MMA), and beta[i] is read only for the columns that pass.  A row without a
+// boost gets what the SAMPLE kernel gives it: its threshold only prunes, the list takes the same exact keys.
+template <int MODE, int STG, int KREG, bool FILTER = false, bool SAMPLE = false, bool BOOST = false>
 __global__ void __launch_bounds__(192, 1) score_stats_kernel(const __grid_constant__ CUtensorMap tmU,
-                                                             const __grid_constant__ CUtensorMap tmE, StatsParams P) {
+                                                             const __grid_constant__ CUtensorMap tmE,
+                                                             std::conditional_t<BOOST, BoostStatsParams, StatsParams> P) {
     constexpr int STAGES = STG;      // (shadows the file-level default)
     extern __shared__ __align__(1024) uint8_t smem_raw[];
     uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
@@ -219,12 +248,30 @@ __global__ void __launch_bounds__(192, 1) score_stats_kernel(const __grid_consta
         uint64_t seed = 0;
         uint32_t nz[4] = {0u, 0u, 0u, 0u}, nz_ctr = 0xFFFFFFFFu;      // (gi >> 2 < 2^29: never a real group)
         if constexpr (SAMPLE) {
-            if (row_ok && P.row_inv_tau[row] != 0.f) { s_a = P.row_inv_tau[row]; s_b = kGumbelMax; seed = P.row_seed[row]; }
+            if (row_ok && (!BOOST || P.row_inv_tau) && P.row_inv_tau[row] != 0.f) {
+                s_a = P.row_inv_tau[row]; s_b = kGumbelMax; seed = P.row_seed[row];
+            }
+        }
+        // BOOST: the row's beta (null: no boost), weight, and bound table at its maxima (w >= 0) or minima (w < 0)
+        const float* brow = nullptr;
+        const float* bext = nullptr;
+        float bw = 0.f;
+        if constexpr (BOOST) {
+            const int bv = row_ok ? P.boost_of_row[row] : -1;
+            if (bv >= 0 && P.row_boost_weight[row] != 0.f) {
+                bw = P.row_boost_weight[row];
+                brow = P.boost + (size_t)bv * P.boost_stride;
+                bext = P.boost_bound + (size_t)bv * P.bound_stride + (bw >= 0.f ? 0 : 1);
+            }
         }
         for (int t = t0, ti = 0; t < t1; ++t, ++ti) {
             const int acc = ti & 1;
             uint32_t aw[8];
             if constexpr (FILTER) tile_allow_words(arow, P.item_offset + t * BN, P.item_offset + P.N, aw);   // in flight during the MMA
+            float bp[8];
+            if constexpr (BOOST) {
+                if (brow) tile_boost_bplus(bext, bw, P.item_offset + t * BN, P.item_offset + P.N, bp);
+            }
             mbar_wait(&bars->tmem_full[acc], (ti >> 1) & 1);
             tc_fence_after();
             const int col0 = t * BN;
@@ -267,10 +314,22 @@ __global__ void __launch_bounds__(192, 1) score_stats_kernel(const __grid_consta
                     // candidate bits first (32 compares), then a compact loop over the few set bits: the insertion
                     // code exists once, not 32 times (instruction-cache footprint), and v[j] is fetched by selects
                     unsigned mbits = 0;
+                    if constexpr (BOOST) {      // one score threshold per chunk, then plain compares
+                        float thr_s = s_b != 0.f ? sample_threshold(thr_v, s_a) : thr_v;
+                        if (brow) {
+                            float b = bp[0];
 #pragma unroll
-                    for (int j = 0; j < 32; ++j) {
-                        if constexpr (SAMPLE) mbits |= (fmaf(v[j], s_a, s_b) >= thr_v) ? (1u << j) : 0u;
-                        else mbits |= (v[j] >= thr_v) ? (1u << j) : 0u;
+                            for (int e = 1; e < 8; ++e) b = (e == c) ? bp[e] : b;
+                            thr_s = boost_threshold(thr_s, b);
+                        }
+#pragma unroll
+                        for (int j = 0; j < 32; ++j) mbits |= (v[j] >= thr_s) ? (1u << j) : 0u;
+                    } else {
+#pragma unroll
+                        for (int j = 0; j < 32; ++j) {
+                            if constexpr (SAMPLE) mbits |= (fmaf(v[j], s_a, s_b) >= thr_v) ? (1u << j) : 0u;
+                            else mbits |= (v[j] >= thr_v) ? (1u << j) : 0u;
+                        }
                     }
                     const int left = n_valid - c * 32;
                     if (left < 32) mbits &= (1u << left) - 1u;
@@ -288,6 +347,9 @@ __global__ void __launch_bounds__(192, 1) score_stats_kernel(const __grid_consta
 #pragma unroll
                         for (int t = 1; t < 32; ++t) x = (t == j) ? v[t] : x;
                         const int lc = c * 32 + j, gi = P.item_offset + col0 + lc;
+                        if constexpr (BOOST) {
+                            if (brow) x = fmaf(bw, __ldg(brow + gi), x);
+                        }
                         if constexpr (SAMPLE) {
                             if (s_b != 0.f) {
                                 const uint32_t ctr = (uint32_t)gi >> 2;
@@ -1010,18 +1072,18 @@ static int pick_topk_splits(int m_tiles, int n_tiles) {
 constexpr size_t kStatsSmem = STAGES * STAGE_BYTES + 256 + 1024;                                        // LSE, register-list top-K
 constexpr size_t kStatsSmemList = STAGES_SMEM_LIST * STAGE_BYTES + 256 + BM * (MAXK_TC + 1) * 8 + 1024;   // shared-memory-list top-K
 
-// Sets the shared-memory limit of every top-K list bucket of one FILTER / SAMPLE flavour (once per process).
-template <bool FILTER, bool SAMPLE>
+// Sets the shared-memory limit of every top-K list bucket of one FILTER / SAMPLE / BOOST flavour (once per process).
+template <bool FILTER, bool SAMPLE, bool BOOST>
 static int topk_set_attrs() {
     static bool attr_set = false;
     if (!attr_set) {
-        HVAE_CUDA(cudaFuncSetAttribute(score_stats_kernel<MODE_TOPK, STAGES, 8, FILTER, SAMPLE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kStatsSmem));
-        HVAE_CUDA(cudaFuncSetAttribute(score_stats_kernel<MODE_TOPK, STAGES, 12, FILTER, SAMPLE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kStatsSmem));
-        HVAE_CUDA(cudaFuncSetAttribute(score_stats_kernel<MODE_TOPK, STAGES, 16, FILTER, SAMPLE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kStatsSmem));
-        HVAE_CUDA(cudaFuncSetAttribute(score_stats_kernel<MODE_TOPK, STAGES, 20, FILTER, SAMPLE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kStatsSmem));
-        HVAE_CUDA(cudaFuncSetAttribute(score_stats_kernel<MODE_TOPK, STAGES, 24, FILTER, SAMPLE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kStatsSmem));
-        HVAE_CUDA(cudaFuncSetAttribute(score_stats_kernel<MODE_TOPK, STAGES, 32, FILTER, SAMPLE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kStatsSmem));
-        HVAE_CUDA(cudaFuncSetAttribute(score_stats_kernel<MODE_TOPK, STAGES_SMEM_LIST, 0, FILTER, SAMPLE>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+        HVAE_CUDA(cudaFuncSetAttribute(score_stats_kernel<MODE_TOPK, STAGES, 8, FILTER, SAMPLE, BOOST>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kStatsSmem));
+        HVAE_CUDA(cudaFuncSetAttribute(score_stats_kernel<MODE_TOPK, STAGES, 12, FILTER, SAMPLE, BOOST>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kStatsSmem));
+        HVAE_CUDA(cudaFuncSetAttribute(score_stats_kernel<MODE_TOPK, STAGES, 16, FILTER, SAMPLE, BOOST>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kStatsSmem));
+        HVAE_CUDA(cudaFuncSetAttribute(score_stats_kernel<MODE_TOPK, STAGES, 20, FILTER, SAMPLE, BOOST>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kStatsSmem));
+        HVAE_CUDA(cudaFuncSetAttribute(score_stats_kernel<MODE_TOPK, STAGES, 24, FILTER, SAMPLE, BOOST>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kStatsSmem));
+        HVAE_CUDA(cudaFuncSetAttribute(score_stats_kernel<MODE_TOPK, STAGES, 32, FILTER, SAMPLE, BOOST>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kStatsSmem));
+        HVAE_CUDA(cudaFuncSetAttribute(score_stats_kernel<MODE_TOPK, STAGES_SMEM_LIST, 0, FILTER, SAMPLE, BOOST>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                        (int)kStatsSmemList));
         attr_set = true;
     }
@@ -1031,19 +1093,20 @@ static int topk_set_attrs() {
 // the list capacity is a compile-time size (register arrays): the smallest bucket that holds K.  A list longer than K costs twice: the
 // admission threshold is its LAST entry (more insertions) and every insertion walks the whole list -- hence buckets at the evaluation
 // protocol's own K values (5, 10, 20: src/ml/evaluate.py k_values)
-template <bool FILTER, bool SAMPLE = false>
-static int launch_topk(int K, dim3 grid, cudaStream_t st, const CUtensorMap& tmU, const CUtensorMap& tmE, const StatsParams& P) {
-    if (int rc = topk_set_attrs<FILTER, SAMPLE>()) return rc;
+template <bool FILTER, bool SAMPLE = false, bool BOOST = false>
+static int launch_topk(int K, dim3 grid, cudaStream_t st, const CUtensorMap& tmU, const CUtensorMap& tmE,
+                       const std::conditional_t<BOOST, BoostStatsParams, StatsParams>& P) {
+    if (int rc = topk_set_attrs<FILTER, SAMPLE, BOOST>()) return rc;
     static const int force_kreg = getenv("HVAE_TOPK_KREG") ? atoi(getenv("HVAE_TOPK_KREG")) : 0;        // A/B runs: a larger bucket than needed
     if (force_kreg >= K && force_kreg <= MAXK_REG) K = force_kreg;       // (P.K, the number of results written, stays)
-    if (K <= 8) launch_pdl(score_stats_kernel<MODE_TOPK, STAGES, 8, FILTER, SAMPLE>, grid, 192, kStatsSmem, st, tmU, tmE, P);
-    else if (K <= 12) launch_pdl(score_stats_kernel<MODE_TOPK, STAGES, 12, FILTER, SAMPLE>, grid, 192, kStatsSmem, st, tmU, tmE, P);
-    else if (K <= 16) launch_pdl(score_stats_kernel<MODE_TOPK, STAGES, 16, FILTER, SAMPLE>, grid, 192, kStatsSmem, st, tmU, tmE, P);
-    else if (K <= 20) launch_pdl(score_stats_kernel<MODE_TOPK, STAGES, 20, FILTER, SAMPLE>, grid, 192, kStatsSmem, st, tmU, tmE, P);
-    else if (K <= 24) launch_pdl(score_stats_kernel<MODE_TOPK, STAGES, 24, FILTER, SAMPLE>, grid, 192, kStatsSmem, st, tmU, tmE, P);
-    else if (K <= MAXK_REG) launch_pdl(score_stats_kernel<MODE_TOPK, STAGES, 32, FILTER, SAMPLE>, grid, 192, kStatsSmem, st, tmU, tmE, P);
-    else launch_pdl(score_stats_kernel<MODE_TOPK, STAGES_SMEM_LIST, 0, FILTER, SAMPLE>, grid, 192, kStatsSmemList, st, tmU, tmE, P);
-    HVAE_LAUNCH_CHECK(SAMPLE ? "tc_score_topk_sampled" : FILTER ? "tc_score_topk_filtered" : "tc_score_topk");
+    if (K <= 8) launch_pdl(score_stats_kernel<MODE_TOPK, STAGES, 8, FILTER, SAMPLE, BOOST>, grid, 192, kStatsSmem, st, tmU, tmE, P);
+    else if (K <= 12) launch_pdl(score_stats_kernel<MODE_TOPK, STAGES, 12, FILTER, SAMPLE, BOOST>, grid, 192, kStatsSmem, st, tmU, tmE, P);
+    else if (K <= 16) launch_pdl(score_stats_kernel<MODE_TOPK, STAGES, 16, FILTER, SAMPLE, BOOST>, grid, 192, kStatsSmem, st, tmU, tmE, P);
+    else if (K <= 20) launch_pdl(score_stats_kernel<MODE_TOPK, STAGES, 20, FILTER, SAMPLE, BOOST>, grid, 192, kStatsSmem, st, tmU, tmE, P);
+    else if (K <= 24) launch_pdl(score_stats_kernel<MODE_TOPK, STAGES, 24, FILTER, SAMPLE, BOOST>, grid, 192, kStatsSmem, st, tmU, tmE, P);
+    else if (K <= MAXK_REG) launch_pdl(score_stats_kernel<MODE_TOPK, STAGES, 32, FILTER, SAMPLE, BOOST>, grid, 192, kStatsSmem, st, tmU, tmE, P);
+    else launch_pdl(score_stats_kernel<MODE_TOPK, STAGES_SMEM_LIST, 0, FILTER, SAMPLE, BOOST>, grid, 192, kStatsSmemList, st, tmU, tmE, P);
+    HVAE_LAUNCH_CHECK(BOOST ? "tc_score_topk_boosted" : SAMPLE ? "tc_score_topk_sampled" : FILTER ? "tc_score_topk_filtered" : "tc_score_topk");
     return 0;
 }
 
@@ -1182,7 +1245,7 @@ int hvae_tc_score_lse_grad(const void* U, int ldu, int B, const void* E, int lde
 static int score_topk(const void* U, int ldu, int B, const void* E, int lde, int N, int d, int item_offset, const int64_t* indptr,
                       const int32_t* indices, const int32_t* rows, const uint32_t* allow, int64_t allow_stride,
                       const int32_t* allow_of_row, const float* row_inv_tau, const uint64_t* row_seed, int K, float* cand_val,
-                      int32_t* cand_idx, void* stream) {
+                      int32_t* cand_idx, void* stream, const BoostArgs* bst = nullptr) {
     if (B == 0) return 0;
     HVAE_REQUIRE(K >= 1 && K <= MAXK_TC, "tc_score_topk: K=%d outside [1,%d]", K, MAXK_TC);
     CUtensorMap tmU, tmE;
@@ -1198,6 +1261,12 @@ static int score_topk(const void* U, int ldu, int B, const void* E, int lde, int
     P.allow = allow; P.allow_stride = allow_stride; P.allow_of_row = allow_of_row;
     P.row_inv_tau = row_inv_tau; P.row_seed = row_seed;
     const dim3 grid(m_tiles, P.n_splits);
+    if (bst) {
+        BoostStatsParams PB{P};
+        PB.boost = bst->boost; PB.boost_stride = bst->boost_stride; PB.boost_bound = bst->bound; PB.bound_stride = bst->bound_stride;
+        PB.boost_of_row = bst->boost_of_row; PB.row_boost_weight = bst->row_weight;
+        return launch_topk<true, true, true>(K, grid, (cudaStream_t)stream, tmU, tmE, PB);
+    }
     if (row_inv_tau) return launch_topk<true, true>(K, grid, (cudaStream_t)stream, tmU, tmE, P);
     if (allow) return launch_topk<true>(K, grid, (cudaStream_t)stream, tmU, tmE, P);
     return launch_topk<false>(K, grid, (cudaStream_t)stream, tmU, tmE, P);
@@ -1243,6 +1312,30 @@ int hvae_tc_score_topk_sampled(const void* U, int ldu, int B, const void* E, int
     }
     return score_topk(U, ldu, B, E, lde, N, d, item_offset, indptr, indices, rows, allow, allow_stride_words, allow_of_row,
                       row_inv_tau, row_seed, K, cand_val, cand_idx, stream);
+}
+
+// Boosted top-K on top of hvae_tc_score_topk_sampled (see the header): rows with a boost rank fmaf(w, beta[i], s), sampled or
+// not; cand_val holds keys.  row_inv_tau / row_seed may be NULL (no row sampled); boost == NULL is hvae_tc_score_topk_sampled,
+// or hvae_tc_score_topk_filtered without row_inv_tau.
+int hvae_tc_score_topk_boosted(const void* U, int ldu, int B, const void* E, int lde, int N, int d, int item_offset,
+                               const int64_t* indptr, const int32_t* indices, const int32_t* rows, const uint32_t* allow,
+                               int64_t allow_stride_words, const int32_t* allow_of_row, const float* row_inv_tau,
+                               const uint64_t* row_seed, const float* boost, int64_t boost_stride, const float* boost_bound,
+                               int64_t bound_stride, const int32_t* boost_of_row, const float* row_boost_weight, int K,
+                               float* cand_val, int32_t* cand_idx, void* stream) {
+    HVAE_REQUIRE(!row_inv_tau || row_seed, "tc_score_topk_boosted: row_inv_tau needs row_seed");
+    if (allow) {
+        HVAE_REQUIRE(allow_of_row, "tc_score_topk_boosted: allow needs allow_of_row");
+        HVAE_REQUIRE(item_offset >= 0 && allow_stride_words >= ((int64_t)item_offset + N + 31) / 32,
+                     "tc_score_topk_boosted: allow_stride_words=%lld does not cover items up to %lld", (long long)allow_stride_words,
+                     (long long)item_offset + N);
+    }
+    const BoostArgs bst{boost, boost_stride, boost_bound, bound_stride, boost_of_row, row_boost_weight};
+    if (boost) {
+        if (int rc = check_boost_args("tc_score_topk_boosted", bst, item_offset, N)) return rc;
+    }
+    return score_topk(U, ldu, B, E, lde, N, d, item_offset, indptr, indices, rows, allow, allow_stride_words, allow_of_row,
+                      row_inv_tau, row_seed, K, cand_val, cand_idx, stream, boost ? &bst : nullptr);
 }
 
 // 1 or 2 numerator sums per (split, row): the pair kernel's two CTAs each report the tiles they owned

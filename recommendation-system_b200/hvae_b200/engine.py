@@ -697,14 +697,17 @@ class Engine:
         ml = self.encode(batch, None)
         return self.latent_and_project(batch.B, ml, None, None, want_kl=False)
 
-    def topk(self, batch: Batch, K: int, exclude_seen=True, item_lo=0, item_hi=None, *, mask=None, allow=None, sample=None):
+    def topk(self, batch: Batch, K: int, exclude_seen=True, item_lo=0, item_hi=None, *, mask=None, allow=None, sample=None,
+             boost=None):
         """Full ranking: scores over items [item_lo,item_hi) -> mask seen -> top-K (value, global index).
 
         mask = (indptr int64 [B+1], indices int32): sorted items to leave out per batch row, used instead of the seen rows
         (exclude_seen is then not looked at).  allow = (bitmaps int32 [F, words], allow_of_row int32 [B]): item allow-sets
         over global ids, -1 = unrestricted.  Slots a filtered row cannot fill hold (-inf, -1).  sample = (inv_tau float32 [B],
         seed int64 [B]): rows with inv_tau != 0 get a Gumbel-top-K draw from softmax(scores * inv_tau), in drawn order, with
-        the drawn items' scores (tc.topk_bf16_from_ub)."""
+        the drawn items' scores (tc.topk_bf16_from_ub).  boost = (table float32 [V, N], bounds (tc.item_boost_bounds),
+        boost_of_row int32 [B], weight float32 [B]): rows with a boost and weight != 0 rank score + weight * table[boost] (then
+        sampled if they are), returned in that order with the chosen items' scores."""
         lay, ws, lib, st = self.lay, self.ws, self.lib, self.stream
         item_hi = lay.N if item_hi is None else item_hi
         n_it = item_hi - item_lo
@@ -714,7 +717,7 @@ class Engine:
         out_idx = torch.empty(B, K, dtype=torch.int32, device=self.dev)
         if self.precision != "fp32":
             from . import tc
-            if tc.topk_bf16(self, batch, u, K, exclude_seen, item_lo, item_hi, out_val, out_idx, mask, allow, sample):
+            if tc.topk_bf16(self, batch, u, K, exclude_seen, item_lo, item_hi, out_val, out_idx, mask, allow, sample, boost):
                 return out_val, out_idx
         csr = batch.csr
         bc = max(1, min(B, (256 * 1024 * 1024) // max(1, n_it)))
@@ -728,7 +731,7 @@ class Engine:
             cv = ws.get("topk_cand_v", (nb, nc * K))
             ci = ws.get("topk_cand_i", (nb, nc * K), torch.int32)
             ov, oi = out_val.data_ptr() + 4 * r0 * K, out_idx.data_ptr() + 4 * r0 * K
-            if mask is None and allow is None and sample is None:
+            if mask is None and allow is None and sample is None and boost is None:
                 lib.mask_topk(p(S), n_it, nb, n_it, item_lo, p(csr.indptr), p(csr.indices), rows_ptr, 1 if exclude_seen else 0, K,
                               p(cv), p(ci), ov, oi, st)
                 continue
@@ -738,14 +741,20 @@ class Engine:
                 indptr_ptr, indices_ptr, excl = p(csr.indptr), p(csr.indices), 1 if exclude_seen else 0
             bm, aor = allow if allow is not None else (None, None)
             aor_ptr = None if aor is None else aor.data_ptr() + 4 * r0
-            if sample is None:
+            if sample is None and boost is None:
                 lib.mask_topk_filtered(p(S), n_it, nb, n_it, item_lo, indptr_ptr, indices_ptr, rows_ptr, excl, p(bm),
                                        0 if bm is None else bm.stride(0), aor_ptr, K, p(cv), p(ci), ov, oi, st)
                 continue
-            lib.mask_topk_sampled(p(S), n_it, nb, n_it, item_lo, indptr_ptr, indices_ptr, rows_ptr, excl, p(bm),
-                                  0 if bm is None else bm.stride(0), aor_ptr, sample[0].data_ptr() + 4 * r0,
-                                  sample[1].data_ptr() + 8 * r0, K, p(cv), p(ci), ov, oi, st)
-            # out_val holds keys: the drawn items' scores, gathered from S (id -1 stays -inf)
+            itau_ptr, seed_ptr = (None, None) if sample is None else (sample[0].data_ptr() + 4 * r0, sample[1].data_ptr() + 8 * r0)
+            if boost is None:
+                lib.mask_topk_sampled(p(S), n_it, nb, n_it, item_lo, indptr_ptr, indices_ptr, rows_ptr, excl, p(bm),
+                                      0 if bm is None else bm.stride(0), aor_ptr, itau_ptr, seed_ptr, K, p(cv), p(ci), ov, oi, st)
+            else:
+                tbl, bnd, bor, bwt = boost
+                lib.mask_topk_boosted(p(S), n_it, nb, n_it, item_lo, indptr_ptr, indices_ptr, rows_ptr, excl, p(bm),
+                                      0 if bm is None else bm.stride(0), aor_ptr, itau_ptr, seed_ptr, p(tbl), tbl.stride(0), p(bnd),
+                                      bnd.stride(0), bor.data_ptr() + 4 * r0, bwt.data_ptr() + 4 * r0, K, p(cv), p(ci), ov, oi, st)
+            # out_val holds keys: the chosen items' scores, gathered from S (id -1 stays -inf)
             sel = out_idx[r0:r0 + nb].long()
             got = S[:nb].gather(1, (sel - item_lo).clamp_(min=0))
             out_val[r0:r0 + nb] = torch.where(sel >= 0, got, torch.full_like(got, float("-inf")))

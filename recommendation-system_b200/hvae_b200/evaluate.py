@@ -22,7 +22,7 @@ from . import data as _data
 from ._cabi import p
 from .engine import Batch, DeviceCSR
 from .model import HybridVAE, create_hybrid_vae
-from .serve import check_seed, check_temperature
+from .serve import check_boost_values, check_boost_weight, check_seed, check_temperature
 
 logger = logging.getLogger(__name__)
 _build_input_matrix = _data.build_input_matrix
@@ -81,6 +81,9 @@ class RecommendationEvaluator:
         # place, so a top-K call that took the pair keeps a consistent table while another thread registers a filter
         self._filters: tuple = (None, {})
         self._filters_lock = threading.Lock()
+        # (float32 [V, n_items] boost table, its block bounds (tc.item_boost_bounds), name -> row): copy-on-write like _filters,
+        # under the same lock
+        self._boosts: tuple = (None, None, {})
 
     # -- item filters ------------------------------------------------------------------------------------------------
     def add_item_filter(self, name: str, item_indices) -> None:
@@ -101,6 +104,45 @@ class RecommendationEvaluator:
                 rows = {**rows, name: 0 if table is None else table.shape[0]}
                 table = row[None] if table is None else torch.cat([table, row[None]])
             self._filters = (table, rows)
+
+    # -- item boosts -------------------------------------------------------------------------------------------------
+    def add_item_boost(self, name: str, values) -> None:
+        """Registers (or replaces) the boost `name`: one finite float32 value per item index, |value| <= 1e6 (serve.MAX_BOOST_VALUE).
+        topk_users(..., boost=name, boost_weight=w) then ranks items by score + w * value (see topk_users)."""
+        vals = check_boost_values(values, self.n_items)
+        from . import tc
+        row = torch.as_tensor(vals, device=self.device)[None]
+        bnd = tc.item_boost_bounds(row)
+        with self._filters_lock:
+            table, bounds, rows = self._boosts
+            if name in rows:
+                table, bounds = table.clone(), bounds.clone()
+                table[rows[name]], bounds[rows[name]] = row[0], bnd[0]
+            else:
+                rows = {**rows, name: 0 if table is None else table.shape[0]}
+                table = row if table is None else torch.cat([table, row])
+                bounds = bnd if bounds is None else torch.cat([bounds, bnd])
+            self._boosts = (table, bounds, rows)
+
+    def item_popularity(self) -> np.ndarray:
+        """int64 [n_items]: the number of interactions of each item in the evaluator's interaction matrix (the usual input of
+        popularity debiasing: add_item_boost(name, -np.log1p(item_popularity())))."""
+        return torch.bincount(self._csr.indices.long(), minlength=self.n_items).cpu().numpy()
+
+    def _boost_params(self, boost, boost_weight, n, boost_row):
+        """-> (boost_of_row int32 [n], weight float32 [n]) host arrays, or None when no user is boosted."""
+        if boost is None:
+            return None
+        names = [boost] * n if isinstance(boost, str) else self._per_user(boost, n, "boost")
+        weights = self._per_user(boost_weight, n, "boost_weight")
+        bor, wt = np.full(n, -1, dtype=np.int32), np.zeros(n, dtype=np.float32)
+        for r, (nm, w) in enumerate(zip(names, weights)):
+            if nm is None:
+                continue
+            if not isinstance(nm, str) or nm not in boost_row:
+                raise ValueError(f"unknown item boost {nm!r}")
+            bor[r], wt[r] = boost_row[nm], np.float32(check_boost_weight(w))
+        return (bor, wt) if (bor >= 0).any() else None
 
     @staticmethod
     def _allow_of_row(item_filter, n, filter_row):
@@ -137,7 +179,7 @@ class RecommendationEvaluator:
 
     # -- batched primitives ----------------------------------------------------------------------------------------
     def topk_users(self, user_indices, top_k: int, exclude_seen: bool = True, *, item_filter=None, exclude=None,
-                   temperature=None, seed=None):
+                   temperature=None, seed=None, boost=None, boost_weight=1.0):
         """(values [n,K] f32, indices [n,K] int32) device tensors for the given users.
 
         item_filter: the name of a filter registered with add_item_filter, or one name (or None) per user: that user only gets
@@ -146,11 +188,20 @@ class RecommendationEvaluator:
         temperature, seed: a scalar or one value per user (None = that user's plain top-K).  A user with a temperature tau
         gets K items drawn without replacement from softmax(scores / tau) over the admissible items (Gumbel-top-K, noise of
         (seed, item): the same arguments give the same draw in any batch and for any K, whose first k items are the k-item
-        draw), in drawn order, with their scores.  tau lies in [1e-3, 1e3], seeds in [0, 2^64); a tau needs a seed."""
+        draw), in drawn order, with their scores.  tau lies in [1e-3, 1e3], seeds in [0, 2^64); a tau needs a seed.
+        boost, boost_weight: the name of a boost registered with add_item_boost (or one name or None per user) and a weight w
+        (a scalar or one per user, a finite real with |w| <= 1e3).  A boosted user's items are ranked by the key
+        fmaf(w, value_i, score_i) (include/hvae_b200.h, hvae_tc_score_topk_boosted), and sampled from softmax(key / tau) if
+        it also has a temperature; the values returned are still the chosen items' model scores."""
         users = torch.as_tensor(np.asarray(user_indices, dtype=np.int32), device=self.device)
         sample = self._sample_params(temperature, seed, users.shape[0])
-        if item_filter is not None or exclude is not None or sample is not None:
-            return self._topk_filtered(users, top_k, exclude_seen, item_filter, exclude, sample)
+        with self._filters_lock:
+            btable, bbounds, boost_row = self._boosts
+        bst = self._boost_params(boost, boost_weight, users.shape[0], boost_row)
+        if bst is not None:
+            bst = (btable, bbounds) + bst
+        if item_filter is not None or exclude is not None or sample is not None or bst is not None:
+            return self._topk_filtered(users, top_k, exclude_seen, item_filter, exclude, sample, bst)
         eng = self.model.engine
         from . import tc
         if eng.precision != "fp32" and exclude_seen and top_k <= tc.MAX_K_REG and users.shape[0] >= 2 * self.batch_users:
@@ -197,7 +248,7 @@ class RecommendationEvaluator:
             seed64[r] = check_seed(sd)
         return (inv_tau, seed64.view(np.int64)) if inv_tau.any() else None
 
-    def _topk_filtered(self, users, top_k, exclude_seen, item_filter, exclude, sample=None):
+    def _topk_filtered(self, users, top_k, exclude_seen, item_filter, exclude, sample=None, boost=None):
         n = users.shape[0]
         with self._filters_lock:
             table, filter_row = self._filters
@@ -213,6 +264,8 @@ class RecommendationEvaluator:
         aor_d = None if aor is None else torch.as_tensor(aor, device=self.device)
         if sample is not None:
             sample = tuple(torch.as_tensor(a, device=self.device) for a in sample)
+        if boost is not None:
+            boost = boost[:2] + tuple(torch.as_tensor(a, device=self.device) for a in boost[2:])
         eng = self.model.engine
         vals, idxs = [], []
         with torch.no_grad():
@@ -221,7 +274,9 @@ class RecommendationEvaluator:
                 mask = None if exclude is None else self._mask_csr(rows, exclude[s:s + rows.shape[0]], exclude_seen)
                 allow = None if aor_d is None else (table, aor_d[s:s + rows.shape[0]].contiguous())
                 smp = None if sample is None else tuple(a[s:s + rows.shape[0]].contiguous() for a in sample)
-                v, i = eng.topk(Batch(self._csr, rows, rows.shape[0], 1), top_k, exclude_seen, mask=mask, allow=allow, sample=smp)
+                bst = None if boost is None else boost[:2] + tuple(a[s:s + rows.shape[0]].contiguous() for a in boost[2:])
+                v, i = eng.topk(Batch(self._csr, rows, rows.shape[0], 1), top_k, exclude_seen, mask=mask, allow=allow, sample=smp,
+                                boost=bst)
                 vals.append(v)
                 idxs.append(i)
         if not vals:

@@ -24,6 +24,9 @@ MAX_TOP_K = 100          # the API's own limit (src/api/server.py: Recommendatio
 # Sampling temperatures: below 1e-3 the draw is the plain top-K wherever scores differ by more than 0.017, above 1e3 it is
 # close to uniform over the admissible items for any trained model; either end is better asked for without a temperature.
 MIN_TEMPERATURE, MAX_TEMPERATURE = 1e-3, 1e3
+# Boosts: |value| <= 1e6 and |weight| <= 1e3 keep |weight * value| <= 1e9, so a boosted key s + w * value stays finite for any
+# finite score (and far from the fp32 range the kernels' bounds work in).
+MAX_BOOST_VALUE, MAX_BOOST_WEIGHT = 1e6, 1e3
 
 
 class UnknownUser(KeyError):
@@ -50,6 +53,29 @@ def check_seed(seed) -> int:
     return seed
 
 
+def check_boost_weight(w) -> float:
+    """A boost weight as float; ValueError unless it is a finite real number with |w| <= MAX_BOOST_WEIGHT."""
+    if isinstance(w, bool) or not isinstance(w, numbers.Real):
+        raise ValueError(f"boost_weight must be a number, got {w!r}")
+    w = float(w)
+    if not (math.isfinite(w) and abs(w) <= MAX_BOOST_WEIGHT):
+        raise ValueError(f"boost_weight must be finite with |boost_weight| <= {MAX_BOOST_WEIGHT:g}, got {w!r}")
+    return w
+
+
+def check_boost_values(values, n_items: int) -> np.ndarray:
+    """Boost values as float32 [n_items]; ValueError unless there is one finite real per item with |value| <= MAX_BOOST_VALUE."""
+    try:
+        v = np.asarray(values, dtype=np.float64)
+    except (TypeError, ValueError) as e:
+        raise ValueError(f"boost values must be real numbers: {e}") from None
+    if v.shape != (n_items,):
+        raise ValueError(f"boost values: expected one value per item ({n_items}), got shape {v.shape}")
+    if not (np.isfinite(v).all() and (np.abs(v) <= MAX_BOOST_VALUE).all()):
+        raise ValueError(f"boost values must be finite with |value| <= {MAX_BOOST_VALUE:g}")
+    return v.astype(np.float32)
+
+
 def _response(user_id, idx: np.ndarray, val: np.ndarray, top_k: int, idx_to_item: dict, total_items: int) -> dict:
     """RecommendationResponse of the reference (server.py:164-178): -inf scores and unmapped items are dropped."""
     recs = []
@@ -60,10 +86,12 @@ def _response(user_id, idx: np.ndarray, val: np.ndarray, top_k: int, idx_to_item
 
 
 def _request_parts(req: tuple) -> tuple:
-    """(user_id, top_k, exclude_seen, item_filter, exclude_items, temperature, seed) of a 3- to 7-element request."""
-    if not 3 <= len(req) <= 7:
-        raise ValueError(f"a request has 3 to 7 elements, got {len(req)}")
-    return tuple(req) + (None,) * (7 - len(req))
+    """(user_id, top_k, exclude_seen, item_filter, exclude_items, temperature, seed, boost, boost_weight) of a 3- to 9-element
+    request (boost_weight None: 1.0)."""
+    if not 3 <= len(req) <= 9:
+        raise ValueError(f"a request has 3 to 9 elements, got {len(req)}")
+    parts = tuple(req) + (None,) * (9 - len(req))
+    return parts[:8] + (1.0 if parts[8] is None else parts[8],)
 
 
 class RecommendService:
@@ -71,14 +99,17 @@ class RecommendService:
     `RecommendationEvaluator.topk_users` (`from_evaluator`).  A launch whose requests use item filters or exclusions calls
     topk_fn(user_indices, K, exclude_seen, item_filter=[name or None per row], exclude=[item index array per row]);
     add_filter_fn(name, item_indices) registers an allow-set with the backend (RecommendationEvaluator.add_item_filter).
-    A launch with sampled requests also passes temperature=[tau or None per row], seed=[seed or None per row]."""
+    A launch with sampled requests also passes temperature=[tau or None per row], seed=[seed or None per row], and one with
+    boosted requests boost=[name or None per row], boost_weight=[w or None per row]; add_boost_fn(name, values float32
+    [n_items]) registers a boost with the backend (RecommendationEvaluator.add_item_boost)."""
 
     def __init__(self, topk_fn: Callable, user_to_idx: dict, idx_to_item: dict, n_items: int, max_batch: int = 4096,
-                 add_filter_fn: Callable | None = None):
+                 add_filter_fn: Callable | None = None, add_boost_fn: Callable | None = None):
         self.topk_fn, self.user_to_idx, self.idx_to_item = topk_fn, user_to_idx, idx_to_item
         self.n_items, self.max_batch = int(n_items), int(max_batch)
-        self.add_filter_fn = add_filter_fn
+        self.add_filter_fn, self.add_boost_fn = add_filter_fn, add_boost_fn
         self.filters: set = set()
+        self.boosts: set = set()
         self._item_to_idx: dict | None = None
         self._seeds = random.Random()         # seeds of sampled requests that bring none (OS entropy)
         self._seeds_lock = threading.Lock()
@@ -88,7 +119,8 @@ class RecommendService:
         def topk(users, K, exclude_seen, **filters):
             v, i = evaluator.topk_users(users, K, exclude_seen, **filters)
             return v.cpu().numpy(), i.cpu().numpy()
-        return cls(topk, evaluator.user_to_idx, idx_to_item, evaluator.n_items, max_batch, evaluator.add_item_filter)
+        return cls(topk, evaluator.user_to_idx, idx_to_item, evaluator.n_items, max_batch, evaluator.add_item_filter,
+                   evaluator.add_item_boost)
 
     def _item_index(self) -> dict:
         if self._item_to_idx is None:
@@ -108,6 +140,31 @@ class RecommendService:
         if self.add_filter_fn is not None:
             self.add_filter_fn(name, idx)
         self.filters.add(name)
+
+    def add_item_boost(self, name: str, values: dict) -> None:
+        """Registers (or replaces) the boost `name` from {API item id: value}; items not listed get 0.  Requests with
+        boost=name and boost_weight=w are then ranked by score + w * value.  Values must be finite with |value| <=
+        MAX_BOOST_VALUE; an id without an item index, or a bad value, raises ValueError and registers nothing."""
+        if not isinstance(name, str):
+            raise ValueError(f"item boost names are strings, got {name!r}")
+        to_idx = self._item_index()
+        try:
+            items = list(values.items())
+        except AttributeError:
+            raise ValueError("item boost values must be a mapping {item id: value}") from None
+        unknown = [i for i, _ in items if i not in to_idx]
+        if unknown:
+            raise ValueError(f"item boost {name!r}: unknown item ids {unknown[:5]}{' ...' if len(unknown) > 5 else ''}")
+        for _, v in items:
+            if isinstance(v, bool) or not isinstance(v, numbers.Real):
+                raise ValueError(f"item boost {name!r}: values must be numbers, got {v!r}")
+        dense = np.zeros(self.n_items, dtype=np.float64)
+        for i, v in items:
+            dense[to_idx[i]] = v
+        dense = check_boost_values(dense, self.n_items)
+        if self.add_boost_fn is not None:
+            self.add_boost_fn(name, dense)
+        self.boosts.add(name)
 
     def _check(self, user_id, top_k, item_filter=None):
         if user_id not in self.user_to_idx:
@@ -134,30 +191,40 @@ class RecommendService:
             return self._seeds.getrandbits(53)       # (exact as a JSON number: a client can send it back unchanged)
 
     def recommend(self, user_id, top_k: int = 10, exclude_seen: bool = True, *, item_filter=None, exclude_items=(),
-                  temperature=None, seed=None) -> dict:
+                  temperature=None, seed=None, boost=None, boost_weight=1.0) -> dict:
         """temperature: None for the top_k best items, else a sampled answer: top_k items drawn without replacement from
         softmax(scores / temperature) (temperature in [MIN_TEMPERATURE, MAX_TEMPERATURE]), in drawn order.  seed: an
         integer in [0, 2^64) (None: the service picks one); the response carries "temperature" and "seed", and the same
-        user, seed, temperature, filter, exclusions and model give the same answer."""
-        out = self.recommend_many([(user_id, top_k, exclude_seen, item_filter, exclude_items, temperature, seed)])[0]
+        user, seed, temperature, filter, exclusions and model give the same answer.
+        boost: the name of a boost registered with add_item_boost; items are then ranked (or, with a temperature, sampled)
+        by score + boost_weight * value (boost_weight a finite real with |w| <= MAX_BOOST_WEIGHT).  "score" stays the
+        model's score; the response carries "boost" and "boost_weight"."""
+        out = self.recommend_many([(user_id, top_k, exclude_seen, item_filter, exclude_items, temperature, seed, boost,
+                                    boost_weight)])[0]
         if isinstance(out, Exception):
             raise out
         return out
 
     def recommend_many(self, requests: Sequence[tuple]) -> list:
-        """requests: (user_id, top_k, exclude_seen[, item_filter[, exclude_items[, temperature[, seed]]]]) tuples.  One launch
-        per exclude_seen group (K = the group's largest top_k), whatever filters, exclusions and temperatures its requests
-        carry.  Exclusions are API item ids; ids without an item index are ignored (they can never be recommended).  A request
-        with a temperature is sampled (see recommend).  Returns, in request order, the response dict or the exception that
-        request would have raised."""
+        """requests: (user_id, top_k, exclude_seen[, item_filter[, exclude_items[, temperature[, seed[, boost[,
+        boost_weight]]]]]]) tuples.  One launch per exclude_seen group (K = the group's largest top_k), whatever filters,
+        exclusions, temperatures and boosts its requests carry.  Exclusions are API item ids; ids without an item index are
+        ignored (they can never be recommended).  A request with a temperature is sampled, one with a boost re-ranked (see
+        recommend).  Returns, in request order, the response dict or the exception that request would have raised."""
         out: list = [None] * len(requests)
         groups: dict[bool, list[int]] = {}
         extra: dict[int, tuple] = {}         # request -> (filter name or None, excluded item indices)
         sampled: dict[int, tuple] = {}       # request -> (temperature, seed)
+        boosted: dict[int, tuple] = {}       # request -> (boost name, weight)
         for n, req in enumerate(requests):
             try:
-                user_id, top_k, exclude_seen, item_filter, exclude_items, temperature, seed = _request_parts(req)
+                user_id, top_k, exclude_seen, item_filter, exclude_items, temperature, seed, boost, boost_weight = \
+                    _request_parts(req)
                 self._check(user_id, top_k, item_filter)
+                if boost is not None:
+                    if not isinstance(boost, str) or boost not in self.boosts:
+                        raise ValueError(f"unknown item boost {boost!r}")
+                    boost_weight = check_boost_weight(boost_weight)
                 excluded = self._excluded(exclude_items)
                 seed = None if seed is None else check_seed(seed)
                 if temperature is not None:
@@ -170,6 +237,8 @@ class RecommendService:
                 extra[n] = (item_filter, excluded)
             if temperature is not None:
                 sampled[n] = (temperature, seed)
+            if boost is not None:
+                boosted[n] = (boost, boost_weight)
             groups.setdefault(bool(exclude_seen), []).append(n)
         for exclude_seen, members in groups.items():
             for s in range(0, len(members), self.max_batch):
@@ -183,12 +252,17 @@ class RecommendService:
                 if any(n in sampled for n in part):
                     kw.update(temperature=[sampled[n][0] if n in sampled else None for n in part],
                               seed=[sampled[n][1] if n in sampled else None for n in part])
+                if any(n in boosted for n in part):
+                    kw.update(boost=[boosted[n][0] if n in boosted else None for n in part],
+                              boost_weight=[boosted[n][1] if n in boosted else None for n in part])
                 val, idx = self.topk_fn(users, K, exclude_seen, **kw)
                 val, idx = np.asarray(val), np.asarray(idx)
                 for r, n in enumerate(part):
                     out[n] = _response(requests[n][0], idx[r], val[r], int(requests[n][1]), self.idx_to_item, self.n_items)
                     if n in sampled:
                         out[n]["temperature"], out[n]["seed"] = sampled[n]
+                    if n in boosted:
+                        out[n]["boost"], out[n]["boost_weight"] = boosted[n]
         return out
 
 
@@ -206,14 +280,16 @@ class MicroBatcher:
         self._thread.start()
 
     def submit(self, user_id, top_k: int = 10, exclude_seen: bool = True, *, item_filter=None, exclude_items=(), temperature=None,
-               seed=None) -> Future:
+               seed=None, boost=None, boost_weight=1.0) -> Future:
         fut: Future = Future()
         if exclude_items is not None and not isinstance(exclude_items, (str, bytes)):
             try:
                 exclude_items = tuple(exclude_items)      # a copy: the caller may reuse its list
             except TypeError:
                 pass                                      # reported for this request by recommend_many
-        if temperature is not None or seed is not None:
+        if boost is not None:
+            req = (user_id, top_k, exclude_seen, item_filter, exclude_items, temperature, seed, boost, boost_weight)
+        elif temperature is not None or seed is not None:
             req = (user_id, top_k, exclude_seen, item_filter, exclude_items, temperature, seed)
         elif item_filter is None and exclude_items in (None, ()):
             req = (user_id, top_k, exclude_seen)

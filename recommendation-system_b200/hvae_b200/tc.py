@@ -74,16 +74,26 @@ def score_loss_bf16(eng, batch, u, want_grad):
     return lse, dot, xsum, O, xsum
 
 
-def topk_bf16(eng, batch, u, K, exclude_seen, item_lo, item_hi, out_val, out_idx, mask=None, allow=None, sample=None) -> bool:
+def topk_bf16(eng, batch, u, K, exclude_seen, item_lo, item_hi, out_val, out_idx, mask=None, allow=None, sample=None,
+              boost=None) -> bool:
     """Fused score + seen-mask + top-K over items [item_lo, item_hi).  False if K is beyond the fused kernel."""
     if K > MAX_K_TC:
         return False
     return topk_bf16_from_ub(eng, batch, user_vectors_bf16(eng, u, batch.B), K, exclude_seen, item_lo, item_hi, out_val, out_idx,
-                             mask, allow, sample)
+                             mask, allow, sample, boost)
+
+
+def rescored_rows(sample, boost):
+    """bool [B]: the rows whose top-K values are keys (sampled, or boosted with a weight != 0), or None when there are none."""
+    rows = None if sample is None else sample[0] != 0
+    if boost is not None:
+        b = (boost[2] >= 0) & (boost[3] != 0)
+        rows = b if rows is None else rows | b
+    return rows
 
 
 def topk_bf16_from_ub(eng, batch, ub, K, exclude_seen, item_lo, item_hi, out_val, out_idx, mask=None, allow=None,
-                      sample=None) -> bool:
+                      sample=None, boost=None) -> bool:
     """The same with the bf16 user vectors [B, r8(d)] already at hand (item-sharded evaluation all-gathers them).
 
     mask = (indptr int64 [B+1], indices int32): items to leave out, one sorted row per BATCH row; it replaces the batch's
@@ -91,7 +101,11 @@ def topk_bf16_from_ub(eng, batch, ub, K, exclude_seen, item_lo, item_hi, out_val
     returns items whose bit is set in bitmaps[allow_of_row[b]] (-1: unrestricted); slots it cannot fill hold (-inf, -1).
     sample = (inv_tau float32 [B], seed int64 [B]): row b with inv_tau[b] != 0 gets a K-item Gumbel-top-K draw from
     softmax(scores / tau) (include/hvae_b200.h, hvae_tc_score_topk_sampled), in drawn order; out_val holds the drawn items'
-    scores.  Rows with inv_tau[b] == 0 get the deterministic top-K."""
+    scores.  Rows with inv_tau[b] == 0 get the deterministic top-K.
+    boost = (table float32 [V, >= N], bounds float32 [V, >= 2 * ceil(N / 32)], boost_of_row int32 [B], weight float32 [B]):
+    row b with boost_of_row[b] >= 0 and weight[b] != 0 ranks fmaf(weight[b], table[boost_of_row[b], i], score_i) (then the
+    Gumbel key of that if sampled; include/hvae_b200.h, hvae_tc_score_topk_boosted); bounds holds (max, min) of each table row
+    over every aligned 32-item block (item_boost_bounds).  out_val holds the chosen items' scores."""
     if K > MAX_K_TC:
         return False
     lay, ws, lib, st = eng.lay, eng.ws, eng.lib, eng.stream
@@ -104,7 +118,16 @@ def topk_bf16_from_ub(eng, batch, ub, K, exclude_seen, item_lo, item_hi, out_val
     ci = ws.get("tc_cand_i", (B, ns * K), torch.int32)
     csr = batch.csr
     with eng.span("score_topk"):
-        if sample is not None:
+        if boost is not None:
+            indptr, indices, rows = (mask[0], mask[1], None) if mask is not None else \
+                ((csr.indptr if exclude_seen else None), csr.indices, batch.rows)
+            bm, aor = allow if allow is not None else (None, None)
+            itau, seed = sample if sample is not None else (None, None)
+            tbl, bnd, bor, bwt = boost
+            lib.tc_score_topk_boosted(p(ub), ld8, B, Eb.data_ptr() + 2 * item_lo * ld8, ld8, n_it, d, item_lo, p(indptr), p(indices),
+                                      p(rows), p(bm), 0 if bm is None else bm.stride(0), p(aor), p(itau), p(seed), p(tbl),
+                                      tbl.stride(0), p(bnd), bnd.stride(0), p(bor), p(bwt), K, p(cv), p(ci), st)
+        elif sample is not None:
             indptr, indices, rows = (mask[0], mask[1], None) if mask is not None else \
                 ((csr.indptr if exclude_seen else None), csr.indices, batch.rows)
             bm, aor = allow if allow is not None else (None, None)
@@ -123,9 +146,23 @@ def topk_bf16_from_ub(eng, batch, ub, K, exclude_seen, item_lo, item_hi, out_val
             lib.tc_score_topk_filtered(p(ub), ld8, B, Eb.data_ptr() + 2 * item_lo * ld8, ld8, n_it, d, item_lo, p(indptr), p(indices),
                                        p(rows), p(bm), 0 if bm is None else bm.stride(0), p(aor), K, p(cv), p(ci), st)
     lib.topk_merge(p(cv), p(ci), B, ns * K, K, p(out_val), p(out_idx), st)
-    if sample is not None:      # sampled rows hold keys: the drawn items' scores, from the same bf16 operands (id -1: -inf)
+    keyed = rescored_rows(sample, boost)
+    if keyed is not None:       # sampled / boosted rows hold keys: the chosen items' scores, from the same bf16 operands (id -1: -inf)
         rank = ws.get("tc_sample_rank", (B,), torch.int32)
         sc = ws.get("tc_sample_score", (B, K))
         lib.candidate_rank(p(ub), ld8, p(Eb), ld8, d, 1, p(out_idx), K, B, p(sc), p(rank), st)
-        torch.where(sample[0][:, None] != 0, sc, out_val, out=out_val)
+        torch.where(keyed[:, None], sc, out_val, out=out_val)
     return True
+
+
+def item_boost_bounds(table):
+    """(max, min) of each row of a float32 boost table [V, N] over every aligned 32-item block -> float32 [V, 2 * ceil(N / 32)]
+    (block j at [2j], [2j + 1]), the pruning bounds of the boosted top-K kernels.  The last block's padding repeats the row's
+    last value, so it changes neither extreme."""
+    V, N = table.shape
+    nb = (N + 31) // 32
+    t = table
+    if nb * 32 != N:
+        t = torch.cat([table, table[:, -1:].expand(V, nb * 32 - N)], dim=1)
+    t = t.reshape(V, nb, 32)
+    return torch.stack([t.amax(dim=2), t.amin(dim=2)], dim=2).reshape(V, 2 * nb).contiguous()
